@@ -2,6 +2,7 @@
 """bench.py — StochGPMP hot-path benchmark (driver contract + tier keys: roofline, cpu_baseline, e2e).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-cuda] [--workload panda|planar]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -18,6 +19,8 @@ e2e      same metric through the public API (StochGPMPBatch.optimize) from HOST 
          read back D2H, both inside the timed region (host clock).  The batch is sharded into --e2e-shards
          StochGPMPBatch objects on their own streams so that a shard's D2H overlaps the next shard's kernel;
          the host waits for every shard at the end of every step.
+dump     --dump-outputs DIR writes what the last timed step returned (see dump_outputs) as DIR/<name>.npy, so that two builds
+         run with the same arguments can be compared output for output: the inputs are seeded and identical from run to run.
 extra    N=1: `configs` (C1 planar as shipped fp64, C2 planar 1024 problems, C3 Panda single problem) and `soft_regime` (C4 at a
          temperature with ESS >> 1: the second RNG sweep of the update is no longer skipped).  N>1: `weak` (4096 problems per
          GPU) and `split` (BASELINE configs[4]: the samples of every particle divided over the N ranks, NCCL all_gather of the
@@ -42,6 +45,7 @@ if ROOT not in sys.path:
 
 METRIC = "trajectory_samples_per_s_per_iteration"
 UNIT = "traj-samples/s"
+DUMP_BYTES = 60 * 10 ** 6           # --dump-outputs stays under 64 MB: a larger batch is sampled by problem
 
 
 # ------------------------------------------------------------------------------------------------ workload
@@ -145,6 +149,7 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        self.proc.wait()
         sm = sorted(float(r[1]) for r in self.rows if len(r) >= 9 and r[1].replace(".", "").isdigit())
         mx = [float(r[2]) for r in self.rows if len(r) >= 9 and r[2].replace(".", "").isdigit()]
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
@@ -294,6 +299,24 @@ def time_steps(pl, obs, steps, warmup, flush=None):
         evs.append((e0, e1))
     torch.cuda.synchronize()
     return sum(a.elapsed_time(b) for a, b in evs) / steps
+
+
+def dump_outputs(out, path):
+    """Write what an optimize() call of a StochGPMPBatch returned, with return_samples=False, as <path>/<name>.npy in the
+    planner's dtype: means_pos / means_vel [B,NP,T,n] (the means the step started from), costs [B,NP,S], grad [B,NP,T,2n].
+    When all B problems exceed DUMP_BYTES, a fixed sample of problems is written (numpy default_rng(0), sorted), the same one
+    for every run with the same batch size."""
+    import numpy as np
+    import torch
+    arrays = {"means_pos": out[0], "means_vel": out[1], "costs": out[4], "grad": out[5]}
+    B = out[0].shape[0]
+    per_problem = sum(a[0].numel() * a.element_size() for a in arrays.values())
+    keep = min(B, DUMP_BYTES // per_problem)
+    idx = np.sort(np.random.default_rng(0).choice(B, keep, replace=False)) if keep < B else np.arange(B)
+    idx = torch.as_tensor(idx, device=out[0].device)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.index_select(0, idx).cpu().numpy())
 
 
 def extra_configs(dev, peaks, flush):
@@ -492,7 +515,7 @@ def run_ours(args, rank, world, local_rank):
         flush.fill_(1.0)                                  # L2 flush (126 MB L2 < 256 MiB), outside the event pair
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        pl.optimize(return_samples=False, **obs)
+        out = pl.optimize(return_samples=False, **obs)
         e1.record()
         evs.append((e0, e1))
     barrier()
@@ -500,6 +523,8 @@ def run_ours(args, rank, world, local_rank):
     launches = _lib.launch_count() - launches0
     clk = clocks.stop() if rank == 0 else None
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)       # before the end-to-end leg, which may run `pl` again
 
     # ---------------- timed: end to end from host buffers ("e2e")
     # Public API only: the batch is sharded into E2E_SHARDS StochGPMPBatch objects (problem_offset keeps every RNG stream where it
@@ -647,10 +672,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs / soft_regime / weak / split blocks")
     ap.add_argument("--e2e-shards", type=int, default=8, help="StochGPMPBatch shards (CUDA streams) per GPU in the end-to-end measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours in a single process")
     if args.impl in ("reference", "reference-cuda"):
         run_reference(args, rank, world)
         return
@@ -668,4 +698,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
     main()

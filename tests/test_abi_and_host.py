@@ -215,15 +215,18 @@ def test_interp_alpha_and_se3_oracle():
 
 
 def test_panda_chain_from_urdf_equals_builtin():
-    """The embedded chain constants == what the reference's URDF says (only where the tree is mounted)."""
+    """The embedded chain constants == what the reference's URDF says: its joints as stored in tests/golden/ and, where a
+    reference checkout is found (oracle/ref_loader.py: $STOCH_GPMP_REF), the original file."""
+    from oracle.ref_loader import reference_root
     from stoch_gpmp_b200.robots import PandaFK, SerialChainFK
-    urdf = "/root/reference/assets/franka_description/robots/panda_arm_no_gripper.urdf"
-    if not os.path.exists(urdf):
-        pytest.skip("reference tree not mounted")
-    a = SerialChainFK.from_urdf(urdf, "panda_link0", "ee_link")
+    urdfs = [os.path.join(ROOT, "tests", "golden", "panda_arm_no_gripper_joints.urdf")]
+    if reference_root() is not None:
+        urdfs.append(os.path.join(reference_root(), "assets", "franka_description", "robots", "panda_arm_no_gripper.urdf"))
     b = PandaFK()
-    assert a.names == b.names and a.joint == b.joint and a.xyz == b.xyz
-    assert np.allclose(np.array(a.R), np.array(b.R), atol=0)
+    for urdf in urdfs:
+        a = SerialChainFK.from_urdf(urdf, "panda_link0", "ee_link")
+        assert a.names == b.names and a.joint == b.joint and a.xyz == b.xyz, urdf
+        assert np.allclose(np.array(a.R), np.array(b.R), atol=0), urdf
     assert b.num_links == 11 and b.n_dofs == 7
 
 
