@@ -606,7 +606,10 @@ static int launch_split_cfg(const sgpmp_shape_t& sh, const CostParams<float>& P,
     constexpr int d = 2 * N, NSTG = SGPMP_SPLIT_NSTG, REC = rec_floats(N);
     const int T = sh.T, M = T * d, Mpad = (M + 3) & ~3, Spad = (sh.S + 3) & ~3, NCH = (sh.S + 31) >> 5;
     const size_t phase_bytes = ((size_t)Mpad + Spad + ((NCH + 4) & ~3)) * 4;
-    const size_t uni = phase_bytes > Cfg::pass1_bytes() ? phase_bytes : Cfg::pass1_bytes();
+    size_t uni = phase_bytes > Cfg::pass1_bytes() ? phase_bytes : Cfg::pass1_bytes();
+    // the union region is also stg_tmp, the 32-float start / goal staging scratch of the kernel's start-up; the state-only form
+    // has no pass-1 region, and with T = 2 and S <= 4 the block phases alone need only 64 or 80 bytes
+    if (uni < 32 * sizeof(float)) uni = 32 * sizeof(float);
     const size_t smem = ((size_t)SPH_SMEM + (size_t)T * REC + Spad + 32 + 32) * sizeof(float) + 32 * sizeof(double) +
                         (size_t)(NB ? ((NA * (2 * NSTG + 1) + 1) & ~1) : 0) * sizeof(uint64_t) + ((uni + 15) & ~(size_t)15);
     if (smem > 227 * 1024) return SGPMP_ERR_UNSUPPORTED;

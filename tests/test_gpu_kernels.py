@@ -617,7 +617,9 @@ def test_fused_problem_sharding_invariance(cuda):
 def test_fused_full_size_properties(cuda):
     """C4 per-problem shape (G=4, K=1, S=512, T=64, n=7, fp32) on a few problems: size-independent
     properties — weights sum to one, grad == sum_s w_s (x_s - mu) on the emitted samples (K4 on the fused
-    kernel's own outputs), determinism, and emitted costs == K3 on the emitted samples."""
+    kernel's own outputs), determinism, and emitted costs == K3 on the emitted samples.  12 particles with S=512 run the
+    single-role kernel in clusters of 8 CTAs (the role-split kernel at this per-problem shape is test_gpu_fused_shapes case d)."""
+    from test_gpu_fused_shapes import expect_kernel
     T, n, G, K, S, B = 64, 7, 4, 1, 512, 3
     dtype = torch.float32
     rs = np.random.RandomState(0)
@@ -635,7 +637,8 @@ def test_fused_full_size_properties(cuda):
     res = []
     for rep in range(2):
         mu = mu0.clone()
-        out = _ops().iterate(sh, low.desc(1.0, sp), tab, 0.1, 1, mu, seed=1, draw0=0, want_samples=True)
+        with expect_kernel(r"iterate_kernel<float, ?2, ?7, ?64, ?1, ?8>"):
+            out = _ops().iterate(sh, low.desc(1.0, sp), tab, 0.1, 1, mu, seed=1, draw0=0, want_samples=True)
         res.append((mu, out))
     (mu1, o1), (mu2, o2) = res
     for k in ('samples', 'costs', 'weights', 'grad'):
@@ -1015,29 +1018,33 @@ torch.save(out, sys.argv[1])
 
 def test_fused_cta_shapes_agree(cuda, tmp_path):
     """The role-split Panda kernel runs as 4 + 4 warps per CTA for large grids (the C4 benchmark) and as 8 + 8 warps for grids of
-    <= 6,144 CTAs (every unit test; the per-GPU share of C4 on 8 GPUs).  $SGPMP_SPLIT_CFG is read once per process, so both shapes
-    run in subprocesses on the same inputs: per-sample costs and samples are bit-identical (a sample's arithmetic does not depend on
-    the CTA shape), weights / gradient / means agree to the rounding of the block-wide softmax sum."""
+    <= 6,144 CTAs (the per-GPU share of C4 on 8 GPUs).  $SGPMP_SPLIT_CFG is read once per process, so both shapes run in
+    subprocesses on the same inputs, 38 problems (152 particles: fewer would run the cluster kernel, which does not read
+    $SGPMP_SPLIT_CFG), and each subprocess checks which kernel ran: per-sample costs and samples are bit-identical (a sample's
+    arithmetic does not depend on the CTA shape), weights / gradient / means agree to the rounding of the block-wide softmax sum."""
     import os
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     script = r'''
-import sys, torch
+import os, sys, torch
 sys.path.insert(0, %r)
+sys.path.insert(0, os.path.join(%r, "tests"))
 import bench
+from test_gpu_fused_shapes import expect_kernel
 dev = torch.device("cuda:0")
-w = bench.workload("panda", 3)
-pl = bench.build_planner(w, 3, dev)
+w = bench.workload("panda", 38)
+pl = bench.build_planner(w, 38, dev)
 obs = {"obstacle_spheres": torch.tensor(w["spheres"], dtype=torch.float32, device=dev)}
-r = pl.optimize(opt_iters=1, return_samples=True, **obs)
+with expect_kernel(r"iterate_split_kernel<7, ?1, ?%%s>" %% sys.argv[2].replace(",", ", ?")):
+    r = pl.optimize(opt_iters=1, return_samples=True, **obs)
 torch.save({"means": pl._means.cpu(), "costs": r[4].cpu(), "samples": r[2].cpu(), "grad": r[5].cpu(), "weights": pl._weights_raw.cpu()}, sys.argv[1])
-''' % root
+''' % (root, root)
     res = []
     for cfg in ("4,4", "8,8"):
         f = str(tmp_path / ("cfg%s.pt" % cfg[0]))
         env = dict(os.environ, SGPMP_SPLIT_CFG=cfg, SGPMP_LOWLAT="0")
-        subprocess.run([sys.executable, "-c", script, f], check=True, env=env, timeout=300)
+        subprocess.run([sys.executable, "-c", script, f, cfg], check=True, env=env, timeout=300)
         res.append(torch.load(f))
     a, b = res
     assert torch.equal(a["costs"], b["costs"]) and torch.equal(a["samples"], b["samples"])
