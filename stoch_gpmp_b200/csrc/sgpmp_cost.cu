@@ -148,11 +148,7 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // DEPTH - 1 steps of HBM latency are covered per thread; every thread copies and reads ONLY ITS OWN slots (lane-consecutive
 // words: conflict-free), so no barrier or mbarrier is involved — cp.async.wait_group orders a thread's own copies.  (A CTA-wide
 // TMA ring with mbarriers was measured SLOWER than the just-in-time loads: profiles/r2/k3_tma_experiment.txt.)
-#ifdef SGPMP_COST_RING_DEPTH      // tuning aid
-template <int N> struct CostRing { static constexpr int DEPTH = SGPMP_COST_RING_DEPTH; };
-#else
 template <int N> struct CostRing { static constexpr int DEPTH = N <= 4 ? 4 : (N <= 7 ? 3 : 2); };
-#endif
 
 template <typename real, int N, int CHAIN>
 __global__ void __launch_bounds__(128)

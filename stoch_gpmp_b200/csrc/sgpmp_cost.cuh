@@ -71,29 +71,23 @@ __device__ __forceinline__ void stage_sphere(const real* s4, real* row, int mode
 
 __device__ __forceinline__ float vsqrt(float x) { return sqrtf(x); }
 __device__ __forceinline__ double vsqrt(double x) { return sqrt(x); }
-__device__ __forceinline__ F2 vsqrt(F2 x) { return f2(sqrtf(lane0(x)), sqrtf(lane1(x))); }
 __device__ __forceinline__ float vmaxv(float a, float b) { return fmaxf(a, b); }
 __device__ __forceinline__ double vmaxv(double a, double b) { return fmax(a, b); }
-__device__ __forceinline__ F2 vmaxv(F2 a, F2 b) { return f2(fmaxf(lane0(a), lane0(b)), fmaxf(lane1(a), lane1(b))); }
 __device__ __forceinline__ float vminv(float a, float b) { return fminf(a, b); }
 __device__ __forceinline__ double vminv(double a, double b) { return fmin(a, b); }
-__device__ __forceinline__ F2 vminv(F2 a, F2 b) { return f2(fminf(lane0(a), lane0(b)), fminf(lane1(a), lane1(b))); }
 __device__ __forceinline__ float vstep_pos(float a) { return a > 0.f ? 1.f : 0.f; }        // 1 where a > 0
 __device__ __forceinline__ double vstep_pos(double a) { return a > 0.0 ? 1.0 : 0.0; }
-__device__ __forceinline__ F2 vstep_pos(F2 a) { return f2(lane0(a) > 0.f ? 1.f : 0.f, lane1(a) > 0.f ? 1.f : 0.f); }
 template <typename V> __device__ __forceinline__ V vneg(V a) { return -a; }
 template <> __device__ __forceinline__ F2 vneg<F2>(F2 a) { return f2(-lane0(a), -lane1(a)); }   // folds into operand modifiers
 
 // Forward kinematics of a serial arm (frames 0..N-1: fixed transform then revolute-z joint f; frames
 // N..n_frames-1 fixed), calling visit(x, y, z) for every link-frame origin in chain order
 // (base first if include_base).  Chain constants come from the kernel-parameter constant bank.
-// V: scalar real or F2 (two samples per thread).
-template <typename V, int N, typename F>
-__device__ __forceinline__ void fk_visit_links(const CostParams<typename VT<V>::real>& P, const V* q, F&& visit) {
-    using real = typename VT<V>::real;
-    const V one = vbroadcast<V>((real)1), zero = vbroadcast<V>((real)0);
-    V R0 = one, R1 = zero, R2 = zero, R3 = zero, R4 = one, R5 = zero, R6 = zero, R7 = zero, R8 = one;
-    V px = zero, py = zero, pz = zero;
+template <typename real, int N, typename F>
+__device__ __forceinline__ void fk_visit_links(const CostParams<real>& P, const real* q, F&& visit) {
+    const real one = 1, zero = 0;
+    real R0 = one, R1 = zero, R2 = zero, R3 = zero, R4 = one, R5 = zero, R6 = zero, R7 = zero, R8 = one;
+    real px = zero, py = zero, pz = zero;
     if (P.include_base) visit(px, py, pz);
     auto fixed = [&](int f) {
         const real* F_ = P.R[f];
@@ -102,18 +96,18 @@ __device__ __forceinline__ void fk_visit_links(const CostParams<typename VT<V>::
         py = vfma(R3, tf[0], vfma(R4, tf[1], vfma(R5, tf[2], py)));
         pz = vfma(R6, tf[0], vfma(R7, tf[1], vfma(R8, tf[2], pz)));
         // R <- R * F
-        const V a0 = vfma(R0, F_[0], vfma(R1, F_[3], R2 * F_[6])), a1 = vfma(R0, F_[1], vfma(R1, F_[4], R2 * F_[7])), a2 = vfma(R0, F_[2], vfma(R1, F_[5], R2 * F_[8]));
-        const V a3 = vfma(R3, F_[0], vfma(R4, F_[3], R5 * F_[6])), a4 = vfma(R3, F_[1], vfma(R4, F_[4], R5 * F_[7])), a5 = vfma(R3, F_[2], vfma(R4, F_[5], R5 * F_[8]));
-        const V a6 = vfma(R6, F_[0], vfma(R7, F_[3], R8 * F_[6])), a7 = vfma(R6, F_[1], vfma(R7, F_[4], R8 * F_[7])), a8 = vfma(R6, F_[2], vfma(R7, F_[5], R8 * F_[8]));
+        const real a0 = vfma(R0, F_[0], vfma(R1, F_[3], R2 * F_[6])), a1 = vfma(R0, F_[1], vfma(R1, F_[4], R2 * F_[7])), a2 = vfma(R0, F_[2], vfma(R1, F_[5], R2 * F_[8]));
+        const real a3 = vfma(R3, F_[0], vfma(R4, F_[3], R5 * F_[6])), a4 = vfma(R3, F_[1], vfma(R4, F_[4], R5 * F_[7])), a5 = vfma(R3, F_[2], vfma(R4, F_[5], R5 * F_[8]));
+        const real a6 = vfma(R6, F_[0], vfma(R7, F_[3], R8 * F_[6])), a7 = vfma(R6, F_[1], vfma(R7, F_[4], R8 * F_[7])), a8 = vfma(R6, F_[2], vfma(R7, F_[5], R8 * F_[8]));
         R0 = a0; R1 = a1; R2 = a2; R3 = a3; R4 = a4; R5 = a5; R6 = a6; R7 = a7; R8 = a8;
     };
 #pragma unroll
     for (int f = 0; f < N; ++f) {
         fixed(f);
         // R <- R * Rz(q_f): col0' = c col0 + s col1, col1' = c col1 - s col0
-        V s, c;
+        real s, c;
         vsincos(q[f], &s, &c);
-        const V n0 = vfma(c, R0, s * R1), n3 = vfma(c, R3, s * R4), n6 = vfma(c, R6, s * R7);
+        const real n0 = vfma(c, R0, s * R1), n3 = vfma(c, R3, s * R4), n6 = vfma(c, R6, s * R7);
         R1 = vfma(c, R1, vneg(s * R0)); R4 = vfma(c, R4, vneg(s * R3)); R7 = vfma(c, R7, vneg(s * R6));
         R0 = n0; R3 = n3; R6 = n6;
         visit(px, py, pz);
@@ -198,41 +192,32 @@ __device__ __noinline__ real ee_se3_cost(const CostParams<real>& P, const real* 
 // remaining translations point, so q[6] is never needed.
 constexpr int PANDA_EVAL_LINKS = 6;   // link3, link4, link5(=link6), link7, link8(=hand), ee
 
-// Joint sin/cos of the STRUCTURED Panda chain (fp32 scalar paths: standalone K3, the low-latency cost kernel, the single-role
-// fused kernel).  1 (default): MUFU sin.approx / cos.approx, as the link warps of the role-split kernel do (sgpmp_cost_pairs.cuh) —
-// these kernels are FMA-pipe bound with an idle XU pipe, and the polynomials are ~21 FMA-pipe instructions per angle; |err| <=
-// 2^-20.9 displaces a link origin by < 5e-7 m (obstacle-dominated costs move by 3e-6 against the fp64 oracle, inside the 1e-5 bar).
-// 0: the polynomial forms of sgpmp_vec.cuh.  The packed (F2) and fp64 instantiations keep vsincos.
-#ifndef SGPMP_FK_MUFU_SINCOS
-#define SGPMP_FK_MUFU_SINCOS 1
-#endif
-template <typename V>
-__device__ __forceinline__ void fk_sincos(V x, V* s, V* c) { vsincos(x, s, c); }
-#if SGPMP_FK_MUFU_SINCOS
-template <>
-__device__ __forceinline__ void fk_sincos<float>(float x, float* s, float* c) { *s = __sinf(x); *c = __cosf(x); }
-#endif
+// Joint sin/cos of the STRUCTURED Panda chain (fp32 only: standalone K3, the low-latency cost kernel, the single-role fused
+// kernel): MUFU sin.approx / cos.approx, as the link warps of the role-split kernel do (sgpmp_cost_pairs.cuh) — these kernels are
+// FMA-pipe bound with an idle XU pipe, and the polynomials of vsincos are ~21 FMA-pipe instructions per angle; |err| <= 2^-20.9
+// displaces a link origin by < 5e-7 m (obstacle-dominated costs move by 3e-6 against the fp64 oracle, inside the 1e-5 bar).
+__device__ __forceinline__ void fk_sincos(float x, float* s, float* c) { *s = __sinf(x); *c = __cosf(x); }
 
-template <typename V>
+template <typename real>
 struct Cols {   // rotation columns a, b, c
-    V ax, ay, az, bx, by, bz, cx, cy, cz;
+    real ax, ay, az, bx, by, bz, cx, cy, cz;
     __device__ __forceinline__ void rot_xp90() {   // R <- R Rx(+90): (a, b, c) -> (a, c, -b)
-        const V tx = bx, ty = by, tz = bz;
+        const real tx = bx, ty = by, tz = bz;
         bx = cx; by = cy; bz = cz;
         cx = vneg(tx); cy = vneg(ty); cz = vneg(tz);
     }
     __device__ __forceinline__ void rot_xm90() {   // R <- R Rx(-90): (a, b, c) -> (a, -c, b)
-        const V tx = bx, ty = by, tz = bz;
+        const real tx = bx, ty = by, tz = bz;
         bx = vneg(cx); by = vneg(cy); bz = vneg(cz);
         cx = tx; cy = ty; cz = tz;
     }
-    __device__ __forceinline__ void rot_z(V q) {  // R <- R Rz(q): a' = c a + s b, b' = c b - s a
-        V s, c;
-        fk_sincos<V>(q, &s, &c);
+    __device__ __forceinline__ void rot_z(real q) {  // R <- R Rz(q): a' = c a + s b, b' = c b - s a
+        real s, c;
+        fk_sincos(q, &s, &c);
         rot_z_sc(s, c);
     }
-    __device__ __forceinline__ void rot_z_sc(V s, V c) {
-        const V nax = vfma(c, ax, s * bx), nay = vfma(c, ay, s * by), naz = vfma(c, az, s * bz);
+    __device__ __forceinline__ void rot_z_sc(real s, real c) {
+        const real nax = vfma(c, ax, s * bx), nay = vfma(c, ay, s * by), naz = vfma(c, az, s * bz);
         bx = vfma(c, bx, vneg(s * ax)); by = vfma(c, by, vneg(s * ay)); bz = vfma(c, bz, vneg(s * az));
         ax = nax; ay = nay; az = naz;
     }
@@ -240,23 +225,22 @@ struct Cols {   // rotation columns a, b, c
 
 // Origins of the 6 q-dependent, distinct link frames of the Panda structure; weights {1,1,2,1,2,1}.
 // o3: origin of the shifted frame (stage_cta_constants); every origin comes out as p - o at no extra instruction.
-template <typename V>
-__device__ __forceinline__ void fk_panda_origins(const CostParams<typename VT<V>::real>& P, const V* q, V (&X)[PANDA_EVAL_LINKS],
-                                                 V (&Y)[PANDA_EVAL_LINKS], V (&Z)[PANDA_EVAL_LINKS], const typename VT<V>::real* o3) {
-    using real = typename VT<V>::real;
+template <typename real>
+__device__ __forceinline__ void fk_panda_origins(const CostParams<real>& P, const real* q, real (&X)[PANDA_EVAL_LINKS],
+                                                 real (&Y)[PANDA_EVAL_LINKS], real (&Z)[PANDA_EVAL_LINKS], const real* o3) {
     // joints 1 and 2 by hand (R starts as the identity; frame 0: t = (0,0,d1); frame 1: t = 0, Rx(-90)):
     //   a = (c1 c0, c1 s0, -s1), b = (-s1 c0, -s1 s0, -c1), c = (-s0, c0, 0),  p = (0, 0, d1)
-    V s0, c0, s1, c1;
-    fk_sincos<V>(q[0], &s0, &c0);
-    fk_sincos<V>(q[1], &s1, &c1);
+    real s0, c0, s1, c1;
+    fk_sincos(q[0], &s0, &c0);
+    fk_sincos(q[1], &s1, &c1);
     const real d1 = P.p[0][2], t2y = P.p[2][1];
-    const V s1c0 = s1 * c0, s1s0 = s1 * s0;
-    V px = vfma(-t2y, s1c0, -o3[0]), py = vfma(-t2y, s1s0, -o3[1]), pz = vfma(-t2y, c1, d1 - o3[2]);          // frame 2: p += t2y * b
+    const real s1c0 = s1 * c0, s1s0 = s1 * s0;
+    real px = vfma(-t2y, s1c0, -o3[0]), py = vfma(-t2y, s1s0, -o3[1]), pz = vfma(-t2y, c1, d1 - o3[2]);          // frame 2: p += t2y * b
     X[0] = px; Y[0] = py; Z[0] = pz;               // link3
     // frame 2 rotation Rx(+90): (a, b, c) -> (a, c, -b)
-    Cols<V> R;
+    Cols<real> R;
     R.ax = c1 * c0; R.ay = c1 * s0; R.az = vneg(s1);
-    R.bx = vneg(s0); R.by = c0; R.bz = vbroadcast<V>((real)0);
+    R.bx = vneg(s0); R.by = c0; R.bz = 0;
     R.cx = s1c0; R.cy = s1s0; R.cz = c1;
     R.rot_z(q[2]);
     px = vfma(P.p[3][0], R.ax, px); py = vfma(P.p[3][0], R.ay, py); pz = vfma(P.p[3][0], R.az, pz);   // frame 3: t = (x,0,0), Rx(+90)
@@ -280,33 +264,32 @@ __device__ __forceinline__ void fk_panda_origins(const CostParams<typename VT<V>
     X[5] = px; Y[5] = py; Z[5] = pz;               // ee_link
 }
 
-template <typename V, int N, int CHAIN = 0>
+template <typename real, int N, int CHAIN = 0>
 struct TrajCost {
-    using real = typename VT<V>::real;
-    V c_start, c_gp, c_goal, c_coll, c_is, c_self, c_ee;
-    V map_pending; // occupancy value gathered at the previous step, not yet accumulated (hides the gather latency)
-    unsigned map_pending_u8;   // byte-map form of it: the RAW byte, converted when consumed (scalar value types)
-    V xp[2 * N];   // previous state
+    real c_start, c_gp, c_goal, c_coll, c_is, c_self, c_ee;
+    real map_pending; // occupancy value gathered at the previous step, not yet accumulated (hides the gather latency)
+    unsigned map_pending_u8;   // byte-map form of it: the RAW byte, converted when consumed
+    real xp[2 * N];   // previous state
 
-    __device__ __forceinline__ void begin() { c_start = c_gp = c_goal = c_coll = c_is = c_self = c_ee = map_pending = vbroadcast<V>((real)0); map_pending_u8 = 0u; }
+    __device__ __forceinline__ void begin() { c_start = c_gp = c_goal = c_coll = c_is = c_self = c_ee = map_pending = (real)0; map_pending_u8 = 0u; }
 
     // Link fields of configuration q (one FK evaluation shared by both):
     //   spheres  sum_l sum_o exp(-0.5 |p_l - c_o|^2 / r_o^2)            LinkDistanceField 'rbf'   costs/fields.py:63-79
     //   self     sum_{i,j} exp(-|p_i - p_j|^2 / (2 margin^2)), all ordered pairs incl. i == j
     //                                                                    LinkSelfDistanceField     costs/fields.py:114-124
-    __device__ __forceinline__ void link_fields(const CostParams<real>& P, const CostSmem<real>& sm, const V* q) {
+    __device__ __forceinline__ void link_fields(const CostParams<real>& P, const CostSmem<real>& sm, const real* q) {
         const int O = P.n_spheres;
-        const V zero = vbroadcast<V>((real)0);
+        const real zero = (real)0;
         if constexpr (CHAIN >= 1) {
             static_assert(N == 7, "Panda structure has 7 joints");
-            V X[PANDA_EVAL_LINKS], Y[PANDA_EVAL_LINKS], Z[PANDA_EVAL_LINKS], PP[PANDA_EVAL_LINKS];
-            fk_panda_origins<V>(P, q, X, Y, Z, sm.sph + SPH_ORIGIN);
+            real X[PANDA_EVAL_LINKS], Y[PANDA_EVAL_LINKS], Z[PANDA_EVAL_LINKS], PP[PANDA_EVAL_LINKS];
+            fk_panda_origins(P, q, X, Y, Z, sm.sph + SPH_ORIGIN);
 #pragma unroll
             for (int l = 0; l < PANDA_EVAL_LINKS; ++l) PP[l] = vfma(X[l], X[l], vfma(Y[l], Y[l], Z[l] * Z[l]));
             // (the sdf / occupancy variants of the sphere field, costs/fields.py:80-86, always take the generic chain code:
             // keeping them out of this path keeps its register footprint at that of the RBF field)
             if (P.has_spheres) {
-                V acc = zero, acc2 = zero;   // acc2: links with weight 2
+                real acc = zero, acc2 = zero;   // acc2: links with weight 2
                 for (int o = 0; o < O; ++o) {
                     const real* s = sm.sph + SPH_STRIDE * o;
                     const real k = s[3];
@@ -314,7 +297,7 @@ struct TrajCost {
                     load4(s + 4, ax, ay, az, b);
 #pragma unroll
                     for (int l = 0; l < PANDA_EVAL_LINKS; ++l) {
-                        const V e = vexp2_fast(vfma(X[l], ax, vfma(Y[l], ay, vfma(Z[l], az, vfma(PP[l], k, b)))));
+                        const real e = vexp2_fast(vfma(X[l], ax, vfma(Y[l], ay, vfma(Z[l], az, vfma(PP[l], k, b)))));
                         if (l == 2 || l == 4) acc2 += e; else acc += e;
                     }
                 }
@@ -324,20 +307,20 @@ struct TrajCost {
                 // weights of the 6 evaluated origins: {1,1,2,1,2,1}; constants: base (w = include_base) and
                 // link1 = link2 at (0,0,z0) (w = 2).  Ordered pairs => every unordered pair counts twice.
                 const real ks = P.self_k, z0 = P.p[0][2];
-                V a1 = zero, a2 = zero, a4 = zero;     // sums of E over unordered pairs with weight product 1, 2, 4
+                real a1 = zero, a2 = zero, a4 = zero;     // sums of E over unordered pairs with weight product 1, 2, 4
 #pragma unroll
                 for (int l = 0; l < PANDA_EVAL_LINKS; ++l) {
                     const bool w2 = (l == 2 || l == 4);
-                    const V e12 = vexp2_fast(ks * vfma((real)-2 * z0, Z[l], PP[l] + z0 * z0));    // vs link1/link2 (w = 2)
+                    const real e12 = vexp2_fast(ks * vfma((real)-2 * z0, Z[l], PP[l] + z0 * z0));    // vs link1/link2 (w = 2)
                     if (w2) a4 += e12; else a2 += e12;
                     if (P.include_base) {
-                        const V eb = vexp2_fast(ks * PP[l]);                                       // vs base (w = 1)
+                        const real eb = vexp2_fast(ks * PP[l]);                                       // vs base (w = 1)
                         if (w2) a2 += eb; else a1 += eb;
                     }
 #pragma unroll
                     for (int m = l + 1; m < PANDA_EVAL_LINKS; ++m) {
-                        const V dx = X[l] - X[m], dy = Y[l] - Y[m], dz = Z[l] - Z[m];
-                        const V e = vexp2_fast(ks * vfma(dx, dx, vfma(dy, dy, dz * dz)));
+                        const real dx = X[l] - X[m], dy = Y[l] - Y[m], dz = Z[l] - Z[m];
+                        const real e = vexp2_fast(ks * vfma(dx, dx, vfma(dy, dy, dz * dz)));
                         const int wp = (w2 ? 2 : 1) * ((m == 2 || m == 4) ? 2 : 1);
                         if (wp == 4) a4 += e; else if (wp == 2) a2 += e; else a1 += e;
                     }
@@ -346,28 +329,28 @@ struct TrajCost {
             }
         } else {
             const int mode = P.sphere_mode;
-            V best = vbroadcast<V>((real)-1e30);      // running max of the sdf variants over links and spheres
-            auto spheres_at = [&](V x, V y, V z, V& acc) {
+            real best = (real)-1e30;      // running max of the sdf variants over links and spheres
+            auto spheres_at = [&](real x, real y, real z, real& acc) {
                 for (int o = 0; o < O; ++o) {
                     const real* s = sm.sph + SPH_STRIDE * o;
-                    const V dx = x - s[0], dy = y - s[1], dz = z - s[2];
-                    const V d2 = vfma(dx, dx, vfma(dy, dy, dz * dz));
+                    const real dx = x - s[0], dy = y - s[1], dz = z - s[2];
+                    const real d2 = vfma(dx, dx, vfma(dy, dy, dz * dz));
                     if (mode == SGPMP_FIELD_RBF) {
                         acc += vexp2_fast(s[3] * d2);
                     } else {
-                        const V sd = s[3] - vsqrt(d2);
+                        const real sd = s[3] - vsqrt(d2);
                         best = vmaxv(best, mode == SGPMP_FIELD_SDF_CLAMPED ? vminv(sd, zero) : sd);
                         acc += vstep_pos(sd);
                     }
                 }
             };
-            auto fold = [&](V acc) { return (mode == SGPMP_FIELD_SDF || mode == SGPMP_FIELD_SDF_CLAMPED) ? best : acc; };
+            auto fold = [&](real acc) { return (mode == SGPMP_FIELD_SDF || mode == SGPMP_FIELD_SDF_CLAMPED) ? best : acc; };
             if (links_interpolated(P)) {
                 // link interpolation (costs/fields.py:68-74, :117-123): keep every origin, append X_i + (X_{i+1} - X_i) alpha_k
                 // for i in [lo, hi) — separately for the two fields, which carry their own (n, range)
-                V PX[SGPMP_MAX_LINK_POINTS], PY[SGPMP_MAX_LINK_POINTS], PZ[SGPMP_MAX_LINK_POINTS];
+                real PX[SGPMP_MAX_LINK_POINTS], PY[SGPMP_MAX_LINK_POINTS], PZ[SGPMP_MAX_LINK_POINTS];
                 int L = 0;
-                fk_visit_links<V, N>(P, q, [&](V x, V y, V z) { PX[L] = x; PY[L] = y; PZ[L] = z; ++L; });
+                fk_visit_links<real, N>(P, q, [&](real x, real y, real z) { PX[L] = x; PY[L] = y; PZ[L] = z; ++L; });
                 auto extend = [&](int n, int lo, int hi, const real* alpha) {
                     int Lx = L;
                     for (int i = lo; i < hi && n > 0; ++i)
@@ -381,40 +364,40 @@ struct TrajCost {
                 };
                 if (P.has_spheres) {
                     const int Lx = extend(P.sphere_interp_n, P.sphere_interp_lo, P.sphere_interp_hi, P.sphere_alpha);
-                    V acc = zero;
+                    real acc = zero;
                     for (int l = 0; l < Lx; ++l) spheres_at(PX[l], PY[l], PZ[l], acc);
                     c_coll += fold(acc);
                 }
                 if (P.has_self) {
                     const int Lx = extend(P.self_interp_n, P.self_interp_lo, P.self_interp_hi, P.self_alpha);
-                    V sa = zero;
+                    real sa = zero;
                     for (int l = 0; l < Lx; ++l)
                         for (int m = l + 1; m < Lx; ++m) {
-                            const V dx = PX[l] - PX[m], dy = PY[l] - PY[m], dz = PZ[l] - PZ[m];
+                            const real dx = PX[l] - PX[m], dy = PY[l] - PY[m], dz = PZ[l] - PZ[m];
                             sa += vexp2_fast(P.self_k * vfma(dx, dx, vfma(dy, dy, dz * dz)));
                         }
                     c_self += (real)2 * sa + (real)Lx;
                 }
             } else if (P.has_self) {
                 // generic chain: keep every origin, then the upper triangle of the pair matrix
-                V PX[SGPMP_MAX_FRAMES + 1], PY[SGPMP_MAX_FRAMES + 1], PZ[SGPMP_MAX_FRAMES + 1];
+                real PX[SGPMP_MAX_FRAMES + 1], PY[SGPMP_MAX_FRAMES + 1], PZ[SGPMP_MAX_FRAMES + 1];
                 int L = 0;
-                V acc = zero;
-                fk_visit_links<V, N>(P, q, [&](V x, V y, V z) {
+                real acc = zero;
+                fk_visit_links<real, N>(P, q, [&](real x, real y, real z) {
                     PX[L] = x; PY[L] = y; PZ[L] = z; ++L;
                     if (P.has_spheres) spheres_at(x, y, z, acc);
                 });
                 if (P.has_spheres) c_coll += fold(acc);
-                V sa = zero;
+                real sa = zero;
                 for (int l = 0; l < L; ++l)
                     for (int m = l + 1; m < L; ++m) {
-                        const V dx = PX[l] - PX[m], dy = PY[l] - PY[m], dz = PZ[l] - PZ[m];
+                        const real dx = PX[l] - PX[m], dy = PY[l] - PY[m], dz = PZ[l] - PZ[m];
                         sa += vexp2_fast(P.self_k * vfma(dx, dx, vfma(dy, dy, dz * dz)));
                     }
                 c_self += (real)2 * sa + (real)L;
             } else {
-                V acc = zero;
-                fk_visit_links<V, N>(P, q, [&](V x, V y, V z) { spheres_at(x, y, z, acc); });
+                real acc = zero;
+                fk_visit_links<real, N>(P, q, [&](real x, real y, real z) { spheres_at(x, y, z, acc); });
                 c_coll += fold(acc);
             }
         }
@@ -430,51 +413,34 @@ struct TrajCost {
         iy = min(max(iy, 0), P.map_w - 1);
         return iy * P.map_w + ix;
     }
-    __device__ __forceinline__ real map_value1(const CostParams<real>& P, const CostSmem<real>& sm, real x, real y) const {
-        const int idx = map_index(P, x, y);
-        if (sm.map_u8) return (real)__ldg(sm.map_u8 + idx);
-        return __ldg(sm.map + idx);
-    }
-    __device__ __forceinline__ V map_value(const CostParams<real>& P, const CostSmem<real>& sm, V x, V y) const {
-        if constexpr (VT<V>::W == 2) {
-            return f2(map_value1(P, sm, vlane(x, 0), vlane(y, 0)), map_value1(P, sm, vlane(x, 1), vlane(y, 1)));
-        } else {
-            return map_value1(P, sm, x, y);
-        }
-    }
 
     // feed state x_t (t = 0..T-1 in order)
     // brow: b_t = (Sigma^-1 mu)_t of this particle (2N reals, 16-byte aligned when 2N % 4 == 0 rows are padded), or null
     // y: x - mu (the IS term is accumulated as mu^T b + y^T b: |y| << |x|, an order of magnitude less fp32 rounding)
     __device__ __forceinline__ void step(const CostParams<real>& P, const CostSmem<real>& sm, int t, int T,
-                                         const V (&x)[2 * N], const V* yp, const V* yv, const real* brow) {
+                                         const real (&x)[2 * N], const real* yp, const real* yv, const real* brow) {
         if (t == 0) {
 #pragma unroll
             for (int j = 0; j < 2 * N; ++j) {
-                const V e = sm.start[j] - x[j];
+                const real e = sm.start[j] - x[j];
                 c_start = vfma(e, e, c_start);
             }
         } else {
 #pragma unroll
             for (int i = 0; i < N; ++i) {
-                const V ep = vfma(-P.dt, xp[N + i], x[i] - xp[i]);
-                const V ev = x[N + i] - xp[N + i];
+                const real ep = vfma(-P.dt, xp[N + i], x[i] - xp[i]);
+                const real ev = x[N + i] - xp[N + i];
                 c_gp = vfma(ep, vfma(P.q12x2, ev, P.q11 * ep), c_gp);
                 c_gp = vfma(P.q22 * ev, ev, c_gp);
             }
             if (P.has_map) {
                 // consume the gather of the PREVIOUS step, issue this step's (integer counts: exact in any order)
-                if constexpr (VT<V>::W == 1) {
-                    if (sm.map_u8) {
-                        c_coll += (real)map_pending_u8;
-                        map_pending_u8 = __ldg(sm.map_u8 + map_index(P, x[0], x[1]));
-                    } else {
-                        c_coll += map_pending;
-                        map_pending = __ldg(sm.map + map_index(P, x[0], x[1]));
-                    }
+                if (sm.map_u8) {
+                    c_coll += (real)map_pending_u8;
+                    map_pending_u8 = __ldg(sm.map_u8 + map_index(P, x[0], x[1]));
                 } else {
                     c_coll += map_pending;
-                    map_pending = map_value(P, sm, x[0], x[1]);
+                    map_pending = __ldg(sm.map + map_index(P, x[0], x[1]));
                 }
             }
             if constexpr (CHAIN >= 0) {        // CHAIN -1: no link fields and no EE goal are compiled in (state-only costs)
@@ -484,7 +450,7 @@ struct TrajCost {
         if (t == T - 1 && P.has_goal) {
 #pragma unroll
             for (int j = 0; j < 2 * N; ++j) {
-                const V e = sm.goal[j] - x[j];
+                const real e = sm.goal[j] - x[j];
                 c_goal = vfma(e, e, c_goal);
             }
         }
@@ -503,7 +469,7 @@ struct TrajCost {
     __device__ __forceinline__ void finish(const CostParams<real>& P, const CostSmem<real>& sm, int T) {
         if (P.has_map) {
             c_coll += map_pending;
-            if constexpr (VT<V>::W == 1) c_coll += (real)map_pending_u8;
+            c_coll += (real)map_pending_u8;
         }
         c_start = c_start * P.inv_sig_start2;
         c_goal = c_goal * P.inv_sig_goal2;
@@ -514,8 +480,8 @@ struct TrajCost {
         c_coll = c_coll * (P.has_map ? P.map_w_coll : P.sphere_w_coll);
         c_self = c_self * P.self_w_coll;
         c_is = (c_is + sm.mub) * P.temperature;
-        // EE SE(3) goal on the last state (xp holds x_{T-1} after the final step); scalar value types only
-        if constexpr (VT<V>::W == 1 && CHAIN >= 0) {
+        // EE SE(3) goal on the last state (xp holds x_{T-1} after the final step)
+        if constexpr (CHAIN >= 0) {
             if (P.has_ee) {
                 real q[N];      // a COPY: taking the address of xp itself would demote the whole previous-state array to local memory
 #pragma unroll
@@ -527,9 +493,9 @@ struct TrajCost {
     // Contribution of ONE time step to the total (everything above is linear in the per-step accumulators): used by the
     // low-latency cost kernel, where a trajectory's time steps are spread over threads.  Call after begin() + step(t) on a fresh
     // object (xp preset to x_{t-1}); the q-independent constants and mu^T b are added by the thread that owns t = T-1.
-    __device__ __forceinline__ V partial(const CostParams<real>& P, const CostSmem<real>& sm, int T, int t) const {
-        V coll = c_coll + map_pending, self = c_self, is = c_is;
-        if constexpr (VT<V>::W == 1) coll = coll + (real)map_pending_u8;
+    __device__ __forceinline__ real partial(const CostParams<real>& P, const CostSmem<real>& sm, int T, int t) const {
+        real coll = c_coll + map_pending, self = c_self, is = c_is;
+        coll = coll + (real)map_pending_u8;
         if (t == T - 1) {
             if (CHAIN >= 1) {
                 coll = coll + (real)(T - 1) * sm.coll_const;
@@ -542,7 +508,7 @@ struct TrajCost {
     }
     // summation order of the shipped examples' cost lists: CostGP (start + gp), CostGoalPrior, self-collision,
     // obstacle collision, EE goal (examples/panda_environment.py:90), then += IS (planner.py:236)
-    __device__ __forceinline__ V total() const { return (((((c_start + c_gp) + c_goal) + c_self) + c_coll) + c_ee) + c_is; }
+    __device__ __forceinline__ real total() const { return (((((c_start + c_gp) + c_goal) + c_self) + c_coll) + c_ee) + c_is; }
 };
 
 // Per-CTA staging of the problem constants into shared memory: start [d], goal [d] of goal index g, the sphere

@@ -14,28 +14,18 @@
 #pragma once
 #include "sgpmp_cost.cuh"
 
-// Joint sin/cos of the packed link-field code: 3 = MUFU sin.approx / cos.approx for all three joint pairs (default), 2 / 1 = only
-// the distal two / one pairs, 0 = the FMA-pipe polynomials of sgpmp_vec.cuh everywhere.  After the role split the link warps are
-// FMA-pipe bound (132 of their 305 instructions per step are packed FP32 holding the pipe for two passes) while the XU pipe idles
-// more than half of the time, and the polynomials were 96 of those FMA cycles.  MUFU's |err| <= 2^-20.9 displaces a link origin by
-// < 5e-7 m; measured where the obstacle term IS the cost (test_fused_link_field_term_dominating, C3 shape, fp32 vs the fp64 oracle):
-// 9.0e-7 / 3.1e-6 with MUFU against 1.9e-7 / 3.3e-6 with the polynomials — inside the 1e-5 bar either way.  C4: 14.59 -> 13.38 ms.
-#ifndef SGPMP_LINK_MUFU_SINCOS
-#define SGPMP_LINK_MUFU_SINCOS 3
-#endif
-
 namespace sgpmp {
-__device__ __forceinline__ void link_sincos(F2 x, F2* s, F2* c, bool mufu) {
-    if (mufu) {
-        *s = f2(__sinf(lane0(x)), __sinf(lane1(x)));
-        *c = f2(__cosf(lane0(x)), __cosf(lane1(x)));
-    } else {
-        vsincos(x, s, c);
-    }
+
+// Joint sin/cos of the packed link-field code: MUFU sin.approx / cos.approx for all three joint pairs.  After the role split the
+// link warps are FMA-pipe bound (132 of their 305 instructions per step are packed FP32 holding the pipe for two passes) while the
+// XU pipe idled more than half of the time, and packed FMA-pipe sin/cos polynomials were 96 of those FMA cycles.  MUFU's
+// |err| <= 2^-20.9 displaces a link origin by < 5e-7 m; measured where the obstacle term IS the cost
+// (test_fused_link_field_term_dominating, C3 shape, fp32 vs the fp64 oracle): 9.0e-7 / 3.1e-6 with MUFU against 1.9e-7 / 3.3e-6
+// with the polynomials — inside the 1e-5 bar either way.  C4: 14.59 -> 13.38 ms.
+__device__ __forceinline__ void link_sincos(F2 x, F2* s, F2* c) {
+    *s = f2(__sinf(lane0(x)), __sinf(lane1(x)));
+    *c = f2(__cosf(lane0(x)), __cosf(lane1(x)));
 }
-}  // namespace sgpmp
-
-namespace sgpmp {
 
 __device__ __forceinline__ float hsum(F2 a) { return lane0(a) + lane1(a); }
 
@@ -64,9 +54,9 @@ struct TrajCostPairs {
         static_assert(CHAIN == 0 || N == 7, "Panda structure has 7 joints");
         if constexpr (CHAIN >= 1) {
             F2 S01, C01, S23, C23, S45, C45;
-            link_sincos(xp[0], &S01, &C01, SGPMP_LINK_MUFU_SINCOS >= 3);
-            link_sincos(xp[1], &S23, &C23, SGPMP_LINK_MUFU_SINCOS >= 2);
-            link_sincos(xp[2], &S45, &C45, SGPMP_LINK_MUFU_SINCOS >= 1);
+            link_sincos(xp[0], &S01, &C01);
+            link_sincos(xp[1], &S23, &C23);
+            link_sincos(xp[2], &S45, &C45);
             const float s0 = lane0(S01), c0 = lane0(C01), s1 = lane1(S01), c1 = lane1(C01);
             // joints 1 and 2 by hand: a = (c1 c0, c1 s0, -s1), b = (-s1 c0, -s1 s0, -c1), c = (-s0, c0, 0), p = (0,0,d1)
             const float d1 = P.p[0][2], t2y = P.p[2][1];

@@ -17,7 +17,6 @@
 //     iterations; particles are independent, so no grid-wide synchronisation exists anywhere.
 //   * FP32-pipe/MUFU bound (DESIGN.md §6); HBM traffic is O(NP*M) per iteration instead of 3*M*S*NP.
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 #include "sgpmp_common.cuh"
 #include "sgpmp_cost.cuh"
@@ -25,44 +24,26 @@
 #include "sgpmp_iterate.cuh"
 #include "sgpmp_rng.cuh"
 
-#ifndef SGPMP_MINB128
-#define SGPMP_MINB128 6       // 6 CTAs x 4 warps at 80 registers: the same 24 warps/SM as 3 x 256 threads, finer block phases
-#endif
-#ifndef SGPMP_MINB256
-#define SGPMP_MINB256 3
-#endif
-#ifndef SGPMP_MINB128_SMALL
-#define SGPMP_MINB128_SMALL 10    // n_dof <= 3 (planar): the whole state is 4-6 registers; 51 registers per thread, 10 CTAs per SM (8: 1.79 ms, 10: 1.77, 12: 1.81)
-#endif
-#ifndef SGPMP_MINB_PACKED
-#define SGPMP_MINB_PACKED 2
-#endif
-#ifndef SGPMP_T_UNROLL
-#define SGPMP_T_UNROLL 1      // unroll factor of the dof-pair time loop (tuning aid; 2 was measured slower, see DESIGN.md §6)
-#endif
-
 namespace cg = cooperative_groups;
-constexpr int SGPMP_T_UNROLL_C = SGPMP_T_UNROLL;
 
 namespace sgpmp {
 
+// fp32 CTAs per SM (__launch_bounds__ minimum blocks)
+constexpr int ITER_MINB256 = 3;
+constexpr int ITER_MINB128 = 6;          // 6 CTAs x 4 warps at 80 registers: the same 24 warps/SM as 3 x 256 threads, finer block phases
+constexpr int ITER_MINB128_SMALL = 10;   // n_dof <= 3 (planar): the whole state is 4-6 registers; 51 registers per thread, 10 CTAs per SM (8: 1.79 ms, 10: 1.77, 12: 1.81)
+
 // PACK selects the pass-1 arithmetic:
 //   0  scalar: one sample per thread (fp32 or fp64)
-//   1  two fp32 samples per thread, packed FFMA2/FADD2/FMUL2 across the two samples (sgpmp_vec.cuh)
 //   2  one fp32 sample per thread, packed arithmetic across neighbouring DoFs / links (sgpmp_cost_pairs.cuh)
-template <typename real, int PACK> struct PackV { using type = real; };
-template <> struct PackV<float, 1> { using type = F2; };
-
 // CL > 1: one particle's S samples are split over a thread-block CLUSTER of CL CTAs (low-latency mode for few
 // problems: B*NP CTAs cannot fill 148 SMs).  Each CTA draws and scores samples [cr*S/CL, (cr+1)*S/CL) with the same
 // global RNG counters; the softmax statistics (max, sum) and the weighted eps-sum are exchanged through distributed
 // shared memory (cluster.map_shared_rank) with four cluster barriers per iteration, then every CTA applies the
 // identical update to its own copy of mu.  No global memory or extra launch is involved.
 template <typename real, int PACK, int N, int BS, int CHAIN, int CL>
-__global__ void __launch_bounds__(BS, (sizeof(real) == 4 ? (PACK == 1 ? SGPMP_MINB_PACKED : (BS == 256 ? SGPMP_MINB256 : ((N <= 3 && CL == 1 && BS == 128) ? SGPMP_MINB128_SMALL : SGPMP_MINB128))) : 1))
+__global__ void __launch_bounds__(BS, (sizeof(real) == 4 ? (BS == 256 ? ITER_MINB256 : ((N <= 3 && CL == 1 && BS == 128) ? ITER_MINB128_SMALL : ITER_MINB128)) : 1))
 iterate_kernel(const __grid_constant__ CostParams<real> P, const __grid_constant__ IterArgs<real> A) {
-    using V = typename PackV<real, PACK>::type;
-    constexpr int W = VT<V>::W;
     constexpr int d = 2 * N;
     constexpr int NP2 = (N + 1) / 2;
     constexpr int VOFF = (PACK == 2) ? 2 * NP2 : N;                   // offset of the velocity half in a shared-memory row
@@ -139,7 +120,7 @@ iterate_kernel(const __grid_constant__ CostParams<real> P, const __grid_constant
                 F2 yp[NP2], yv[NP2];
 #pragma unroll
                 for (int k = 0; k < NP2; ++k) yp[k] = yv[k] = f2(0.f, 0.f);
-#pragma unroll SGPMP_T_UNROLL_C
+#pragma unroll 1                        // 2 was measured slower (DESIGN.md §6)
                 for (int t = 0; t < T; ++t) {
                     F2 ep[NP2], ev[NP2];
                     if (eps) {
@@ -186,41 +167,30 @@ iterate_kernel(const __grid_constant__ CostParams<real> P, const __grid_constant
                 if (last && A.costs) A.costs[(size_t)bp * S + s0] = c;
             }
         } else {
-            for (int k = tid; s_lo + k * W < s_hi; k += BS) {
-                const int s0 = s_lo + k * W;                               // lane 0 sample; lane 1 (packed) is s0 + 1
-                const int s1 = (W == 2 && s0 + 1 < s_hi) ? s0 + 1 : s0;    // odd count: the last lane 1 shadows lane 0
-                TrajCost<V, N, CHAIN> tc;
+            for (int s0 = s_lo + tid; s0 < s_hi; s0 += BS) {
+                TrajCost<real, N, CHAIN> tc;
                 tc.begin();
-                V yp[N], yv[N];
+                real yp[N], yv[N];
     #pragma unroll
-                for (int i = 0; i < N; ++i) { yp[i] = vbroadcast<V>((real)0); yv[i] = vbroadcast<V>((real)0); }
-                // One Philox call per DoF (and lane) yields the normals of TWO time steps; the step body is kept as a
+                for (int i = 0; i < N; ++i) { yp[i] = 0; yv[i] = 0; }
+                // One Philox call yields the four normals of a DoF pair; the step body is kept as a
                 // single (not 2x unrolled) copy so that the hot loop stays inside the instruction cache.
     #pragma unroll 1
                 for (int t = 0; t < T; ++t) {
-                    V e[d + 1];
+                    real e[d + 1];
                     if (eps) {
     #pragma unroll
                         for (int j = 0; j < d; ++j) {
                             const real* row = eps + ((size_t)t * d + j) * S;
-                            if constexpr (W == 2) e[j] = f2(row[s0], row[s1]); else e[j] = row[s0];
+                            e[j] = row[s0];
                         }
                     } else {
     #pragma unroll
                         for (int k = 0; k < (N + 1) / 2; ++k) {
-                            constexpr int NN = N;
-                            const bool full = (2 * k + 1 < NN);
-                            if constexpr (W == 2) {
-                                float a0, a1, a2, a3, b0, b1, b2, b3;
-                                normal_pair<float>(key, (uint32_t)t, (uint32_t)k, full, A.sample_gid0 + (uint32_t)s0, pgid, a0, a1, a2, a3, dro);
-                                normal_pair<float>(key, (uint32_t)t, (uint32_t)k, full, A.sample_gid0 + (uint32_t)(s0 + 1), pgid, b0, b1, b2, b3, dro);
-                                e[2 * k] = f2(a0, b0); e[N + 2 * k] = f2(a2, b2);
-                                if (full) { e[2 * k + 1] = f2(a1, b1); e[N + 2 * k + 1] = f2(a3, b3); }
-                            } else {
-                                real p1, v1;
-                                normal_pair<real>(key, (uint32_t)t, (uint32_t)k, full, A.sample_gid0 + (uint32_t)s0, pgid, e[2 * k], p1, e[N + 2 * k], v1, dro);
-                                if (full) { e[2 * k + 1] = p1; e[N + 2 * k + 1] = v1; }
-                            }
+                            const bool full = (2 * k + 1 < N);
+                            real p1, v1;
+                            normal_pair<real>(key, (uint32_t)t, (uint32_t)k, full, A.sample_gid0 + (uint32_t)s0, pgid, e[2 * k], p1, e[N + 2 * k], v1, dro);
+                            if (full) { e[2 * k + 1] = p1; e[N + 2 * k + 1] = v1; }
                         }
                     }
                     real r[8], m[DP];
@@ -228,11 +198,11 @@ iterate_kernel(const __grid_constant__ CostParams<real> P, const __grid_constant
                     load4(tabGH + t * 8 + 4, r[4], r[5], r[6], r[7]);
     #pragma unroll
                     for (int q = 0; q < DP / 4; ++q) load4(mu + t * DP + 4 * q, m[4 * q], m[4 * q + 1], m[4 * q + 2], m[4 * q + 3]);
-                    V x[d];
+                    real x[d];
     #pragma unroll
                     for (int i = 0; i < N; ++i) {
-                        const V np_ = vfma(r[0], e[i], vneg(vfma(r[3], yp[i], r[4] * yv[i])));
-                        const V nv_ = vfma(r[1], e[i], r[2] * e[N + i]) - vfma(r[5], yp[i], r[6] * yv[i]);
+                        const real np_ = vfma(r[0], e[i], vneg(vfma(r[3], yp[i], r[4] * yv[i])));
+                        const real nv_ = vfma(r[1], e[i], r[2] * e[N + i]) - vfma(r[5], yp[i], r[6] * yv[i]);
                         yp[i] = np_; yv[i] = nv_;
                         x[i] = m[i] + np_;
                         x[N + i] = m[N + i] + nv_;
@@ -242,19 +212,14 @@ iterate_kernel(const __grid_constant__ CostParams<real> P, const __grid_constant
     #pragma unroll
                         for (int j = 0; j < d; ++j) {
                             real* row = A.samples + ((size_t)bp * M + (size_t)t * d + j) * S;
-                            row[s0] = vlane(x[j], 0);
-                            if (W == 2 && s1 != s0) row[s1] = vlane(x[j], 1);
+                            row[s0] = x[j];
                         }
                     }
                 }
                 tc.finish(P, sm, T);
-                const V c = tc.total();
-                wsm[s0 - s_lo] = vlane(c, 0);
-                if (last && A.costs) A.costs[(size_t)bp * S + s0] = vlane(c, 0);
-                if (W == 2 && s1 != s0) {
-                    wsm[s1 - s_lo] = vlane(c, 1);
-                    if (last && A.costs) A.costs[(size_t)bp * S + s1] = vlane(c, 1);
-                }
+                const real c = tc.total();
+                wsm[s0 - s_lo] = c;
+                if (last && A.costs) A.costs[(size_t)bp * S + s0] = c;
             }
         }
         __syncthreads();
@@ -439,54 +404,42 @@ static int launch_iterate_nb(const sgpmp_shape_t& sh, const CostParams<real>& P,
 // few problems: split every particle's samples over a cluster of 8 / 4 / 2 CTAs (DSMEM reductions) so that the
 // launch still covers the 148 SMs: the largest cluster that keeps <= 2 CTAs per SM and >= 64 samples per CTA
 static int iterate_cluster_size(const sgpmp_shape_t& sh, bool injected_eps) {
-    static const char* cl_env = getenv("SGPMP_ITERATE_CLUSTER");    // 0 disables
     const long n_part = (long)sh.B * sh.G * sh.K;
-    if ((cl_env && atoi(cl_env) == 0) || injected_eps) return 1;
+    if (injected_eps) return 1;
     for (int c = 8; c >= 2; c >>= 1)
         if (n_part * c <= 2 * 148 && sh.S >= 64 * c && (c == 8 ? sh.S >= 256 : true)) return c;
     return 1;
 }
 
-template <typename real, int N, int CHAIN>
-static int launch_iterate_n(const sgpmp_shape_t& sh, const CostParams<real>& P, const IterArgs<real>& A, cudaStream_t st) {
-    static const char* force_bs = getenv("SGPMP_ITERATE_BS");       // tuning aids
-    static const char* pack_env = getenv("SGPMP_ITERATE_PACK");     // 0 scalar, 2 dof pairs (default)
-    const bool bs128 = force_bs && atoi(force_bs) == 128;
-    const long n_part = (long)sh.B * sh.G * sh.K;
+// fp32 dof-pair pass 1 (PACK 2): the Panda structure (CHAIN 1, 2) and, with CHAIN 0, costs without link fields (occupancy map or
+// no obstacle cost).  Cluster mode for few problems.
+template <int N, int CHAIN>
+static int launch_iterate_pairs(const sgpmp_shape_t& sh, const CostParams<float>& P, const IterArgs<float>& A, cudaStream_t st) {
     const int cl = A.stats_out ? 1 : iterate_cluster_size(sh, A.eps_in != nullptr);
+    if (cl == 8) return launch_iterate_nb<float, 2, N, 64, CHAIN, 8>(sh, P, A, st);
+    if (cl == 4) return launch_iterate_nb<float, 2, N, 128, CHAIN, 4>(sh, P, A, st);
+    if (cl == 2) return launch_iterate_nb<float, 2, N, 128, CHAIN, 2>(sh, P, A, st);
+    // CTA size.  Chains with link fields (Panda): 256 threads, 3 CTAs/SM.  (128 threads at 6 CTAs/SM — the same 24 warps per SM —
+    // measured 17.19 against 17.41 ms at 4096 problems, but 1.65 against 1.20 ms at 256 problems and 4.80 against 4.56 ms at 1024:
+    // each CTA then runs twice as long, so the last partial wave costs more than the finer block phases gain.)  Without link fields
+    // (planar: a short per-sample body, so the per-iteration block phases — b = P mu, softmax, update — weigh more and 80 registers
+    // are not needed) 128-thread CTAs at 10 CTAs/SM and 48 registers give 2.23 -> 1.81 ms at 4096 x 4 x 256; grids too small to
+    // fill that keep 256 threads.
+    const long n_part = (long)sh.B * sh.G * sh.K;
+    const bool light = (CHAIN == 0) && !(P.has_spheres || P.has_self);
+    if (sh.S > 128 && !(light && n_part >= 10L * 148)) return launch_iterate_nb<float, 2, N, 256, CHAIN>(sh, P, A, st);
+    return launch_iterate_nb<float, 2, N, 128, CHAIN>(sh, P, A, st);
+}
+
+// every cost list without the Panda structure: dof pairs where they apply, else the scalar pass 1 (fp64, generic FK chains,
+// the other DoF counts)
+template <typename real, int N>
+static int launch_iterate_n(const sgpmp_shape_t& sh, const CostParams<real>& P, const IterArgs<real>& A, cudaStream_t st) {
     if constexpr (sizeof(real) == 4 && (N == 2 || N == 7)) {
-        const bool pairs_ok_c = ((CHAIN >= 1) || !(P.has_spheres || P.has_self)) && !(P.has_spheres && P.sphere_mode != SGPMP_FIELD_RBF);
-        if (pairs_ok_c) {
-            if (cl == 8) return launch_iterate_nb<real, 2, N, 64, CHAIN, 8>(sh, P, A, st);
-            if (cl == 4) return launch_iterate_nb<real, 2, N, 128, CHAIN, 4>(sh, P, A, st);
-            if (cl == 2) return launch_iterate_nb<real, 2, N, 128, CHAIN, 2>(sh, P, A, st);
-        }
+        if (!(P.has_spheres || P.has_self)) return launch_iterate_pairs<N, 0>(sh, P, A, st);
     }
-    if constexpr (sizeof(real) == 4 && (N == 2 || N == 7)) {
-        const int pack = pack_env ? atoi(pack_env) : 2;
-        // dof-pair packing covers the occupancy-map field and the Panda structure; generic FK chains stay scalar
-        const bool pairs_ok = ((CHAIN >= 1) || !(P.has_spheres || P.has_self)) && !(P.has_spheres && P.sphere_mode != SGPMP_FIELD_RBF);
-        if (pack == 2 && pairs_ok) {
-            // CTA size.  Chains with link fields (Panda): 256 threads, 3 CTAs/SM.  (128 threads at 6 CTAs/SM — the same 24 warps
-            // per SM — measured 17.19 against 17.41 ms at 4096 problems, but 1.65 against 1.20 ms at 256 problems and 4.80 against
-            // 4.56 ms at 1024: each CTA then runs twice as long, so the last partial wave costs more than the finer block phases
-            // gain.  SGPMP_ITERATE_BS=128 selects it.)  Without link fields (planar: a short per-sample body, so the per-iteration
-            // block phases — b = P mu, softmax, update — weigh more and 80 registers are not needed) 128-thread CTAs at 10 CTAs/SM
-            // and 48 registers give 2.23 -> 1.81 ms at 4096 x 4 x 256; grids too small to fill that keep 256 threads.
-            const bool light = (CHAIN == 0) && !(P.has_spheres || P.has_self);
-            const bool want128 = bs128 || (light && n_part >= 10L * 148);
-            if (sh.S > 128 && !want128) return launch_iterate_nb<real, 2, N, 256, CHAIN>(sh, P, A, st);
-            return launch_iterate_nb<real, 2, N, 128, CHAIN>(sh, P, A, st);
-        }
-#ifdef SGPMP_ENABLE_TWO_SAMPLE_PACKING   // measured 4 % slower than dof pairs (register pressure); kept for experiments
-        if (pack == 1) {
-            if (sh.S > 256 && !bs128) return launch_iterate_nb<real, 1, N, 256, CHAIN>(sh, P, A, st);
-            return launch_iterate_nb<real, 1, N, 128, CHAIN>(sh, P, A, st);
-        }
-#endif
-    }
-    if (sh.S > 128 && !bs128) return launch_iterate_nb<real, 0, N, 256, CHAIN>(sh, P, A, st);
-    return launch_iterate_nb<real, 0, N, 128, CHAIN>(sh, P, A, st);
+    if (sh.S > 128) return launch_iterate_nb<real, 0, N, 256, 0>(sh, P, A, st);
+    return launch_iterate_nb<real, 0, N, 128, 0>(sh, P, A, st);
 }
 
 template <typename real>
@@ -509,27 +462,24 @@ static int launch_iterate(const sgpmp_shape_t& sh, const sgpmp_cost_desc_t& desc
     A.costs = (real*)costs; A.weights = (real*)weights; A.grad = (real*)grad;
     A.stats_out = (real*)stats_out;
     if constexpr (sizeof(real) == 4) {
+        // the role-split kernel (sgpmp_iterate_split.cu) unless the grid is small enough for cluster mode; the single-role
+        // kernel also takes the shapes it does not support (T < 2, shared memory beyond 227 KiB at large S)
+        const bool split = A.stats_out || iterate_cluster_size(sh, A.eps_in != nullptr) == 1;
         if (structured_fields_ok(P) && chain_is_panda_structure(desc, sh.n_dof)) {
-            // Panda structure: role-split kernel (sgpmp_iterate_split.cu) unless the grid is small enough for cluster mode
-            static const char* split_env = getenv("SGPMP_ITERATE_SPLIT");     // 0 selects the single-role kernel
-            if (!(split_env && atoi(split_env) == 0) && (A.stats_out || iterate_cluster_size(sh, A.eps_in != nullptr) == 1)) {
+            if (split) {
                 rc = launch_iterate_split(sh, P, A, P.has_self ? 2 : 1, st);
                 if (rc != SGPMP_ERR_UNSUPPORTED) return rc;
             }
-            return P.has_self ? launch_iterate_n<real, 7, 2>(sh, P, A, st) : launch_iterate_n<real, 7, 1>(sh, P, A, st);
+            return P.has_self ? launch_iterate_pairs<7, 2>(sh, P, A, st) : launch_iterate_pairs<7, 1>(sh, P, A, st);
         }
-    }
-    if constexpr (sizeof(real) == 4) {
         // no link fields (planar occupancy map / no obstacle cost): the state-only form of the record-layout kernel
-        static const char* split_env = getenv("SGPMP_ITERATE_SPLIT");
-        if (!(split_env && atoi(split_env) == 0) && !(P.has_spheres || P.has_self || P.has_ee) &&
-            (A.stats_out || iterate_cluster_size(sh, A.eps_in != nullptr) == 1)) {
+        if (split && !(P.has_spheres || P.has_self || P.has_ee)) {
             rc = launch_iterate_split(sh, P, A, 0, st);
             if (rc != SGPMP_ERR_UNSUPPORTED) return rc;
         }
     }
     switch (sh.n_dof) {
-#define SGPMP_DOF_CASE(N) case N: return launch_iterate_n<real, N, 0>(sh, P, A, st);
+#define SGPMP_DOF_CASE(N) case N: return launch_iterate_n<real, N>(sh, P, A, st);
 #include "sgpmp_dof_list.inc"
 #undef SGPMP_DOF_CASE
         default:

@@ -17,8 +17,6 @@
 // instructions are spills, RNG and FK compete for the same registers and instruction cache).  Split, each role
 // fits 64 registers without spills, the SM holds 32 warps instead of 24, and the scheduler always has an ALU/XU
 // stream (Philox, Box-Muller) next to an FMA/XU stream (chain, RBF) to pick from.  See DESIGN.md §4.2.
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "sgpmp_common.cuh"
@@ -27,29 +25,10 @@
 #include "sgpmp_iterate.cuh"
 #include "sgpmp_rng.cuh"
 
-#ifndef SGPMP_SPLIT_TS
-#define SGPMP_SPLIT_TS 5        // time steps per ring stage (C4: 1 / 2 / 3 / 4 / 5 steps 13.77 / 13.62 / 13.32 / 13.21 / 13.11 ms; 6 no longer fits four CTAs per SM)
-#endif
-#ifndef SGPMP_SPLIT_NSTG
-#define SGPMP_SPLIT_NSTG 2      // ring stages per warp pair
-#endif
-#ifndef SGPMP_SPLIT_MINB
-#define SGPMP_SPLIT_MINB 4      // CTAs per SM at 256 threads (64 registers)
-#endif
-#ifndef SGPMP_SPLIT_UNROLL_A
-#define SGPMP_SPLIT_UNROLL_A 1  // unroll factor of the state warps' step loop
-#endif
-#ifndef SGPMP_SPLIT_UNROLL_B
-#define SGPMP_SPLIT_UNROLL_B 1  // unroll factor of the link warps' step loop
-#endif
-#ifndef SGPMP_SPLIT_SLEEP_NS
-#define SGPMP_SPLIT_SLEEP_NS 64 // back-off of a warp that finds its mbarrier phase incomplete (form without the suspend-time hint)
-#endif
-#ifndef SGPMP_SPLIT_WAIT_HINT_NS
-#define SGPMP_SPLIT_WAIT_HINT_NS 1000   // suspend-time hint of mbarrier.try_wait; 0 selects the try_wait + nanosleep form
-#endif
-
 namespace sgpmp {
+
+constexpr int SPLIT_TS = 5;     // time steps per ring stage (C4: 1 / 2 / 3 / 4 / 5 steps 13.77 / 13.62 / 13.32 / 13.21 / 13.11 ms; 6 no longer fits four CTAs per SM)
+constexpr int SPLIT_NSTG = 2;   // ring stages per warp pair
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -59,13 +38,13 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 // Wait until the phase of the given parity has completed (a fresh barrier has "completed" parity 1).  A warp that has to
-// wait is SUSPENDED (try_wait with a suspend-time hint, or nanosleep between polls): a spinning warp would spend the issue
-// slots the other role needs (first version: 7 % of all executed instructions were this loop).
+// wait is SUSPENDED: a spinning warp would spend the issue slots the other role needs (first version: 7 % of all executed
+// instructions were this loop).  The hardware suspends the warp inside try_wait for up to the hinted time, so no instructions
+// run between polls.  Measured at C4 (profiles/r2/wait_variants.txt): hint 1000 / 20000 ns 13.15 ms, try_wait + nanosleep
+// 64 / 256 / 1000 / 4000 ns 13.21-13.22 ms — the wait loop is not what bounds the kernel (a waiting warp only uses issue slots
+// nobody else had a use for).
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-#if SGPMP_SPLIT_WAIT_HINT_NS > 0
-    // the hardware suspends the warp inside try_wait for up to the hinted time: no instructions between polls.  Measured at C4
-    // (profiles/r2/wait_variants.txt): hint 1000 / 20000 ns 13.15 ms, try_wait + nanosleep 64 / 256 / 1000 / 4000 ns 13.21-13.22 ms —
-    // the wait loop is not what bounds the kernel (a waiting warp only uses issue slots nobody else had a use for)
+    constexpr uint32_t HINT_NS = 1000;
     asm volatile(
         "{\n"
         ".reg .pred P1;\n"
@@ -74,21 +53,8 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
         "@P1 bra DONE;\n"
         "bra LAB_WAIT;\n"
         "DONE:\n"
-        "}" ::"r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)SGPMP_SPLIT_WAIT_HINT_NS)
+        "}" ::"r"(smem_u32(bar)), "r"(parity), "r"(HINT_NS)
         : "memory");
-#else
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-        "@P1 bra DONE;\n"
-        "nanosleep.u32 %2;\n"
-        "bra LAB_WAIT;\n"
-        "DONE:\n"
-        "}" ::"r"(smem_u32(bar)), "r"(parity), "n"(SGPMP_SPLIT_SLEEP_NS)
-        : "memory");
-#endif
 }
 
 __device__ __forceinline__ F2 ld_f2(const float* p) { const float2 v = *reinterpret_cast<const float2*>(p); return f2(v.x, v.y); }
@@ -108,16 +74,17 @@ constexpr int REC_G = 0, REC_B = 4, REC_M = 8;
 __host__ __device__ constexpr int rec_floats(int n_dof) { return 8 + 12 * ((n_dof + 1) / 2); }
 __device__ __forceinline__ int rec_col(int i, int a, int what) { return 8 + 12 * (i >> 1) + what + 2 * a + (i & 1); }   // a: 0 pos, 1 vel
 
-// NA state warps + NB link warps per CTA (NA % NB == 0): 32 NA samples per sweep; link warp j serves the state warps
-// j, j + NB, ... stage by stage.  NB = 0: no link fields (CHAIN = 0; the planar occupancy-map cost is gathered by the state
-// warps themselves) — then there is no ring and no mbarrier, just the state role with its record layout.
+// NA state warps + NB link warps per CTA: 32 NA samples per sweep.  NB = NA: state warp w feeds link warp w.  NB = 0: no link
+// fields (CHAIN = 0; the planar occupancy-map cost is gathered by the state warps themselves) — then there is no ring and no
+// mbarrier, just the state role with its record layout.
 template <int NA, int NB> struct SplitCfg {
+    static_assert(NB == 0 || NB == NA, "one link warp per state warp");
     static constexpr int BS = 32 * (NA + NB), SW = 32 * NA;
     // CTAs per SM: with link warps as many as 1024 threads (64 registers each) allow; state-only CTAs fit 48 registers
-    static constexpr int MINB = NB ? ((1024 / BS) > 0 ? (1024 / BS) : 1) : (1280 / BS > 24 ? 24 : 1280 / BS);
+    static constexpr int MINB = NB ? 1024 / BS : (1280 / BS > 24 ? 24 : 1280 / BS);
     // shared-memory bytes of the region that pass 1 uses for the ring + link sums and the block phases for acc / nzl / nzo
     __host__ __device__ static constexpr size_t pass1_bytes() {
-        return NB ? (size_t)NA * SGPMP_SPLIT_NSTG * SGPMP_SPLIT_TS * 96 * sizeof(float2) + (size_t)32 * NA * 8 * sizeof(float) : 0;
+        return NB ? (size_t)NA * SPLIT_NSTG * SPLIT_TS * 96 * sizeof(float2) + (size_t)32 * NA * 8 * sizeof(float) : 0;
     }
 };
 
@@ -125,13 +92,12 @@ template <int N, int CHAIN, int NA, int NB>
 __global__ void __launch_bounds__(SplitCfg<NA, NB>::BS, SplitCfg<NA, NB>::MINB)
 iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_constant__ IterArgs<float> A) {
     using Cfg = SplitCfg<NA, NB>;
-    constexpr int d = 2 * N, NP2 = (N + 1) / 2, REC = rec_floats(N), BS = Cfg::BS, SW = Cfg::SW, R = NB ? NA / (NB ? NB : 1) : 0;
-    static_assert(NB == 0 || NA % (NB ? NB : 1) == 0, "every link warp serves the same number of state warps");
+    constexpr int d = 2 * N, NP2 = (N + 1) / 2, REC = rec_floats(N), BS = Cfg::BS, SW = Cfg::SW;
     static_assert((CHAIN == 0) == (NB == 0), "link warps exist exactly when the chain has link fields");
     static_assert(CHAIN == 0 || N == 7, "Panda structure has 7 joints");
     static_assert(NP2 <= 4, "start / goal staging holds up to 8 DoF");
-    constexpr int TS = NB ? SGPMP_SPLIT_TS : 16;      // state-only form: a 'stage' is just the span of the two-level GP sum
-    constexpr int NSTG = SGPMP_SPLIT_NSTG, UNROLL_A = SGPMP_SPLIT_UNROLL_A, UNROLL_B = SGPMP_SPLIT_UNROLL_B;
+    constexpr int TS = NB ? SPLIT_TS : 16;      // state-only form: a 'stage' is just the span of the two-level GP sum
+    constexpr int NSTG = SPLIT_NSTG;
     constexpr int SLOT = 3 * 32;                                      // float2 per (state warp, step): q pairs 0..2 x 32 lanes
     const int T = A.T, S = A.S, G = A.G, K = A.K;
     const int M = T * d, Mpad = (M + 3) & ~3, Spad = (S + 3) & ~3, NCH = (S + 31) >> 5;
@@ -190,10 +156,6 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
     sm.map_u8 = (P.has_map && P.occ_map_u8) ? P.occ_map_u8 + (size_t)(P.map_of_problem ? P.map_of_problem[b] : 0) * P.map_h * P.map_w : nullptr;
     __syncthreads();
 
-#ifdef SGPMP_SPLIT_STAGGER_NS
-    // de-phase the state warps of a CTA (identical instruction streams started together keep hitting the same pipe together)
-    if (role == 0 && wa > 0) __nanosleep(wa * SGPMP_SPLIT_STAGGER_NS);
-#endif
     const int ns = S;
     const int n_sweeps = (ns + SW - 1) / SW;
     uint32_t sc = 0;      // ring stages used so far (identical in both roles)
@@ -314,7 +276,7 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
                     float2* slot = NB > 0 ? ring + ((size_t)(wa * NSTG + stg) * TS) * SLOT + lane : nullptr;
                     const float* blk = rec + t0 * REC;
                     F2 cgs = f2(0.f, 0.f);          // GP sum of this stage (two-level accumulation)
-#pragma unroll UNROLL_A
+#pragma unroll 1
                     for (int t = t0; t < tend; ++t, slot += SLOT, blk += REC) {
                         F2 ep[NP2], ev[NP2];
                         draw(t, ep, ev);
@@ -408,70 +370,33 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
               }
             } else if constexpr (NB > 0) {
                 // ================= link warps =================
-                // per stage: the R state warps this warp serves, in turn; the stage's link-field sums are folded into the
-                // shared-memory accumulators of (state warp, lane) — a fixed order, so results do not depend on timing.
-                // The sweep is instantiated for the common sphere counts as compile-time constants (oc = 0: run-time loop).
+                // Link warp wb serves state warp wb.  The field sums of the whole sweep stay in registers and reach shared memory
+                // once, at the end (folding them into shared memory per stage cost ~16 instructions per stage on the warps that
+                // are the critical path).  The sweep is instantiated for the common sphere counts as compile-time constants
+                // (oc = 0: run-time loop).
                 auto link_sweep = [&](auto oc) {
                     constexpr int OC = decltype(oc)::value;
-                    if constexpr (R == 1) {
-                        // one state warp per link warp (every shipped configuration): the field sums of the whole sweep stay in
-                        // registers and reach shared memory once, at the end (the per-stage fold of the general form below costs
-                        // ~16 instructions per stage on the warps that are the critical path)
-                        const int w = wb;
-                        TrajCostPairs<N, CHAIN> tc;
-                        tc.begin();
-                        for (int t0 = 1; t0 < T; t0 += TS) {
-                            const uint32_t stg = sc % NSTG, use = sc / NSTG;
-                            const int tend = min(t0 + TS, T);
-                            mbar_wait(bar_full(w, stg), use & 1u);
-                            const float2* slot = ring + ((size_t)(w * NSTG + stg) * TS) * SLOT + lane;
-#pragma unroll UNROLL_B
-                            for (int t = t0; t < tend; ++t, slot += SLOT) {
-                                F2 xq[NP2];
-                                xq[0] = ld_f2(slot); xq[1] = ld_f2(slot + 32); xq[2] = ld_f2(slot + 64);
-                                xq[3] = f2(0.f, 0.f);
-                                tc.template link_fields<OC>(P, sm, xq);
-                            }
-                            mbar_arrive(bar_empty(w, stg));
-                            ++sc;
-                        }
-                        float4* ba = reinterpret_cast<float4*>(bacc + (size_t)(w * 32 + lane) * 8);
-                        ba[0] = make_float4(lane0(tc.a01), lane1(tc.a01), lane0(tc.a23), lane1(tc.a23));
-                        ba[1] = make_float4(lane0(tc.a45), lane1(tc.a45), tc.c_self, 0.f);
-                        mbar_arrive(bar_res(w));                         // the sums of the sweep are complete
-                        return;
-                    }
+                    TrajCostPairs<N, CHAIN> tc;
+                    tc.begin();
                     for (int t0 = 1; t0 < T; t0 += TS) {
                         const uint32_t stg = sc % NSTG, use = sc / NSTG;
                         const int tend = min(t0 + TS, T);
+                        mbar_wait(bar_full(wb, stg), use & 1u);
+                        const float2* slot = ring + ((size_t)(wb * NSTG + stg) * TS) * SLOT + lane;
 #pragma unroll 1
-                        for (int j = 0; j < R; ++j) {
-                            const int w = wb + j * NB;
-                            mbar_wait(bar_full(w, stg), use & 1u);
-                            const float2* slot = ring + ((size_t)(w * NSTG + stg) * TS) * SLOT + lane;
-                            TrajCostPairs<N, CHAIN> tc;
-                            tc.begin();
-#pragma unroll 1
-                            for (int t = t0; t < tend; ++t, slot += SLOT) {
-                                F2 xq[NP2];
-                                xq[0] = ld_f2(slot); xq[1] = ld_f2(slot + 32); xq[2] = ld_f2(slot + 64);
-                                xq[3] = f2(0.f, 0.f);
-                                tc.template link_fields<OC>(P, sm, xq);
-                            }
-                            float4* ba = reinterpret_cast<float4*>(bacc + (size_t)(w * 32 + lane) * 8);
-                            float4 v0 = make_float4(lane0(tc.a01), lane1(tc.a01), lane0(tc.a23), lane1(tc.a23));
-                            float4 v1 = make_float4(lane0(tc.a45), lane1(tc.a45), tc.c_self, 0.f);
-                            if (t0 != 1) {
-                                const float4 o0 = ba[0], o1 = ba[1];
-                                v0.x += o0.x; v0.y += o0.y; v0.z += o0.z; v0.w += o0.w;
-                                v1.x += o1.x; v1.y += o1.y; v1.z += o1.z;
-                            }
-                            ba[0] = v0; ba[1] = v1;
-                            mbar_arrive(bar_empty(w, stg));
-                            if (tend == T) mbar_arrive(bar_res(w));      // last stage of the sweep: the sums are complete
+                        for (int t = t0; t < tend; ++t, slot += SLOT) {
+                            F2 xq[NP2];
+                            xq[0] = ld_f2(slot); xq[1] = ld_f2(slot + 32); xq[2] = ld_f2(slot + 64);
+                            xq[3] = f2(0.f, 0.f);
+                            tc.template link_fields<OC>(P, sm, xq);
                         }
+                        mbar_arrive(bar_empty(wb, stg));
                         ++sc;
                     }
+                    float4* ba = reinterpret_cast<float4*>(bacc + (size_t)(wb * 32 + lane) * 8);
+                    ba[0] = make_float4(lane0(tc.a01), lane1(tc.a01), lane0(tc.a23), lane1(tc.a23));
+                    ba[1] = make_float4(lane0(tc.a45), lane1(tc.a45), tc.c_self, 0.f);
+                    mbar_arrive(bar_res(wb));                            // the sums of the sweep are complete
                 };
                 const int n_sph = P.has_spheres ? P.n_spheres : -1;
                 if (n_sph == 5) link_sweep(std::integral_constant<int, 5>{});          // examples/panda_environment.py:125-133
@@ -603,7 +528,7 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
 template <int N, int CHAIN, int NA, int NB>
 static int launch_split_cfg(const sgpmp_shape_t& sh, const CostParams<float>& P, const IterArgs<float>& A, cudaStream_t st) {
     using Cfg = SplitCfg<NA, NB>;
-    constexpr int d = 2 * N, NSTG = SGPMP_SPLIT_NSTG, REC = rec_floats(N);
+    constexpr int d = 2 * N, NSTG = SPLIT_NSTG, REC = rec_floats(N);
     const int T = sh.T, M = T * d, Mpad = (M + 3) & ~3, Spad = (sh.S + 3) & ~3, NCH = (sh.S + 31) >> 5;
     const size_t phase_bytes = ((size_t)Mpad + Spad + ((NCH + 4) & ~3)) * 4;
     size_t uni = phase_bytes > Cfg::pass1_bytes() ? phase_bytes : Cfg::pass1_bytes();
@@ -623,32 +548,23 @@ static int launch_split_cfg(const sgpmp_shape_t& sh, const CostParams<float>& P,
 
 template <int CHAIN>
 static int launch_split_chain(const sgpmp_shape_t& sh, const CostParams<float>& P, const IterArgs<float>& A, cudaStream_t st) {
-    static const char* cfg_env = getenv("SGPMP_SPLIT_CFG");       // tuning aid: "NA,NB"
     // equal numbers of state and link warps measured best at C4 (4,4: 14.55 ms; 4,2: 15.7; 8,4: 15.6; 4,1: 20.4; 6,2: 20.2)
-    int na = sh.S > 64 ? 4 : (sh.S > 32 ? 2 : 1), nb = na;
     // Mid-size batches (the 4096-problem config sharded over 8 GPUs: 2,048 CTAs): 512-thread CTAs, two per SM.  The same 32 warps
     // per SM, but a CTA takes half as long, so the partial last wave costs half as much (ms per iteration, (4,4) -> (8,8):
     // 128 problems 0.529 -> 0.502, 256: 0.920 -> 0.861, 512: 1.721 -> 1.699, 1024: 3.417 -> 3.370; 4096: 13.25 -> 13.32, where
     // the finer interleave of four CTAs' block phases wins instead).
     const long n_cta = (long)sh.B * sh.G * sh.K;
-    if (sh.S >= 256 && n_cta <= 6144) na = nb = 8;
-    if (cfg_env) sscanf(cfg_env, "%d,%d", &na, &nb);
-#define SGPMP_SPLIT_CASE(a, b) if (na == a && nb == b) return launch_split_cfg<7, CHAIN, a, b>(sh, P, A, st);
-    SGPMP_SPLIT_CASE(4, 4) SGPMP_SPLIT_CASE(2, 2) SGPMP_SPLIT_CASE(1, 1) SGPMP_SPLIT_CASE(4, 2) SGPMP_SPLIT_CASE(8, 4) SGPMP_SPLIT_CASE(8, 8)
-#undef SGPMP_SPLIT_CASE
-    set_error("sgpmp_iterate(split): configuration %d,%d is not instantiated", na, nb);
-    return SGPMP_ERR_INVALID_ARG;
+    if (sh.S >= 256 && n_cta <= 6144) return launch_split_cfg<7, CHAIN, 8, 8>(sh, P, A, st);
+    if (sh.S > 64) return launch_split_cfg<7, CHAIN, 4, 4>(sh, P, A, st);
+    if (sh.S > 32) return launch_split_cfg<7, CHAIN, 2, 2>(sh, P, A, st);
+    return launch_split_cfg<7, CHAIN, 1, 1>(sh, P, A, st);
 }
 
 // state-only form (no link fields): n_dof 2, 3, 4, 6 — the planar occupancy-map cost or no obstacle cost at all
 template <int N>
 static int launch_state_only(const sgpmp_shape_t& sh, const CostParams<float>& P, const IterArgs<float>& A, cudaStream_t st) {
-    static const char* na_env = getenv("SGPMP_STATE_WARPS");      // tuning aid: state warps per CTA (1, 2, 4, 8)
-    int na = sh.S > 64 ? 4 : (sh.S > 32 ? 2 : 1);
-    if (na_env) na = atoi(na_env);
-    if (na == 8) return launch_split_cfg<N, 0, 8, 0>(sh, P, A, st);
-    if (na == 4) return launch_split_cfg<N, 0, 4, 0>(sh, P, A, st);
-    if (na == 2) return launch_split_cfg<N, 0, 2, 0>(sh, P, A, st);
+    if (sh.S > 64) return launch_split_cfg<N, 0, 4, 0>(sh, P, A, st);
+    if (sh.S > 32) return launch_split_cfg<N, 0, 2, 0>(sh, P, A, st);
     return launch_split_cfg<N, 0, 1, 0>(sh, P, A, st);
 }
 

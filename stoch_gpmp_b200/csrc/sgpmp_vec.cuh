@@ -1,14 +1,15 @@
-// Value types of the per-sample arithmetic: scalar `float` / `double`, or `F2` = two fp32 samples packed in one
-// 64-bit register pair and processed with sm_100's packed-FP32 instructions (PTX add/sub/mul/fma .f32x2 ->
-// SASS FADD2 / FMUL2 / FFMA2).
+// Packed fp32 arithmetic: `F2` = two fp32 values in one 64-bit register pair, processed with sm_100's packed-FP32
+// instructions (PTX add/sub/mul/fma .f32x2 -> SASS FADD2 / FMUL2 / FFMA2).  The two halves hold the same quantity of two
+// neighbouring DoFs (2k, 2k+1) of ONE trajectory sample, or of two neighbouring links of the sphere field
+// (sgpmp_cost_pairs.cuh, the role-split fused kernel).
 //
 // Why: the fused kernel is bound by the single issue port of each SM sub-partition (1 warp instruction per
 // clock), not by the FP32 lanes: FFMA2 performs two FMAs per lane per ISSUED instruction (it occupies the FMA
 // pipe for two passes, so peak FLOP/s is unchanged — measured 70.6 TFLOP/s for both forms) and frees every
 // second FP issue slot for the integer (Philox), MUFU and LDS instructions of the same warp
 // (profiles/r1/ffma2_probe.txt: 128 FFMA + 64 LOP3 = 4.25 ms, 64 FFMA2 + 64 LOP3 = 3.37 ms).
-// One thread therefore owns TWO trajectory samples (lanes .x / .y).  Scalars broadcast for free: ptxas turns
-// pack(s, s) into the `R.F32` broadcast operand form, and lane extraction is register-pair aliasing.
+// Scalars broadcast for free: ptxas turns pack(s, s) into the `R.F32` broadcast operand form, and lane extraction is
+// register-pair aliasing.  The scalar overloads below (float / double) serve the one-sample-per-thread code.
 #pragma once
 #include "sgpmp_common.cuh"
 
@@ -37,12 +38,6 @@ __device__ __forceinline__ F2 operator*(F2 a, float s) { return a * f2(s, s); }
 __device__ __forceinline__ F2 operator*(float s, F2 a) { return f2(s, s) * a; }
 __device__ __forceinline__ F2& operator+=(F2& a, F2 b) { a = a + b; return a; }
 
-// ---- uniform interface over scalar and packed values -------------------------------------------------
-template <typename V> struct VT;
-template <> struct VT<float>  { using real = float;  static constexpr int W = 1; };
-template <> struct VT<double> { using real = double; static constexpr int W = 1; };
-template <> struct VT<F2>     { using real = float;  static constexpr int W = 2; };
-
 // a * b + c in one rounding
 __device__ __forceinline__ float vfma(float a, float b, float c) { return fmaf(a, b, c); }
 __device__ __forceinline__ double vfma(double a, double b, double c) { return fma(a, b, c); }
@@ -53,25 +48,16 @@ __device__ __forceinline__ F2 vfma(F2 a, F2 b, float c) { return vfma(a, b, f2(c
 __device__ __forceinline__ F2 vfma(float a, F2 b, float c) { return vfma(f2(a, a), b, f2(c, c)); }
 __device__ __forceinline__ F2 vfma(F2 a, float b, float c) { return vfma(a, f2(b, b), f2(c, c)); }
 
-template <typename V> __device__ __forceinline__ V vbroadcast(typename VT<V>::real s);
-template <> __device__ __forceinline__ float vbroadcast<float>(float s) { return s; }
-template <> __device__ __forceinline__ double vbroadcast<double>(double s) { return s; }
-template <> __device__ __forceinline__ F2 vbroadcast<F2>(float s) { return f2(s, s); }
-
-__device__ __forceinline__ float vlane(float a, int) { return a; }
-__device__ __forceinline__ double vlane(double a, int) { return a; }
-__device__ __forceinline__ float vlane(F2 a, int k) { return k ? lane1(a) : lane0(a); }
-
 // 2^x (fp32: ex2.approx) / e^x (fp64) — the RBF kernels pre-scale their exponent accordingly
 __device__ __forceinline__ float vexp2_fast(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ double vexp2_fast(double x) { return exp(x); }
 __device__ __forceinline__ F2 vexp2_fast(F2 x) { return f2(vexp2_fast(lane0(x)), vexp2_fast(lane1(x))); }
 
-// sin/cos of joint angles.  fp32: branch-free on the FMA pipe — x = j pi + r with j = rint(x / pi) (magic-number rounding,
+// sin/cos of joint angles of the generic FK chain (fk_visit_links).  fp32: branch-free on the FMA pipe — x = j pi + r with j = rint(x / pi) (magic-number rounding,
 // two-term Cody-Waite), sin x = (-1)^j sin r, cos x = (-1)^j cos r, minimax polynomials on |r| <= pi/2 (max abs error
 // 1.2e-7 on |x| <= 4.5, the fp32 rounding floor of values near 1).  Reducing by pi instead of pi/2 costs two more
 // polynomial terms but removes the quadrant swap: the sign is ONE xor per output with the parity bit of the magic
-// sum.  Packed form: 16 FFMA2/FMUL2/FADD2 + 6 integer ops per angle PAIR.  fp64: libdevice.
+// sum.  fp64: libdevice.
 __device__ __forceinline__ void vsincos(double x, double* s, double* c) { sincos(x, s, c); }
 #define SGPMP_SIN_C0 -0.1666666716337204f
 #define SGPMP_SIN_C1 0.008333331905305386f
@@ -95,19 +81,6 @@ __device__ __forceinline__ void vsincos(float x, float* sp, float* cp) {
     const float c = fmaf(fmaf(fmaf(fmaf(fmaf(SGPMP_COS_C4, z, SGPMP_COS_C3), z, SGPMP_COS_C2), z, SGPMP_COS_C1), z, SGPMP_COS_C0), z, 1.0f);
     *sp = __uint_as_float(__float_as_uint(s) ^ sb);
     *cp = __uint_as_float(__float_as_uint(c) ^ sb);
-}
-__device__ __forceinline__ void vsincos(F2 x, F2* sp, F2* cp) {
-    const F2 t = vfma(x, 0.3183098861837907f, 12582912.0f);
-    const unsigned sb0 = __float_as_uint(lane0(t)) << 31, sb1 = __float_as_uint(lane1(t)) << 31;
-    const F2 j = t - 12582912.0f;
-    F2 r = vfma(j, -3.1415927410125732f, x);
-    r = vfma(j, 8.742277657347586e-08f, r);
-    const F2 z = r * r;
-    const F2 ps = vfma(vfma(vfma(vfma(f2(SGPMP_SIN_C4, SGPMP_SIN_C4), z, SGPMP_SIN_C3), z, SGPMP_SIN_C2), z, SGPMP_SIN_C1), z, SGPMP_SIN_C0) * z;
-    const F2 s = vfma(ps, r, r);
-    const F2 c = vfma(vfma(vfma(vfma(vfma(f2(SGPMP_COS_C4, SGPMP_COS_C4), z, SGPMP_COS_C3), z, SGPMP_COS_C2), z, SGPMP_COS_C1), z, SGPMP_COS_C0), z, 1.0f);
-    *sp = f2(__uint_as_float(__float_as_uint(lane0(s)) ^ sb0), __uint_as_float(__float_as_uint(lane1(s)) ^ sb1));
-    *cp = f2(__uint_as_float(__float_as_uint(lane0(c)) ^ sb0), __uint_as_float(__float_as_uint(lane1(c)) ^ sb1));
 }
 
 }  // namespace sgpmp

@@ -277,7 +277,7 @@ def five_checks(case, kernel, claims=(), cost_tol=TOL_F32, problems=None):
 # ------------------------------------------------------------------------------------------------ role-split Panda kernel
 # (B, G, S, T, O, self, EE, shared spheres, expected kernel, claimed terms)
 PANDA_CASES = {
-    # 1+1 warps, one ragged sweep, 3 ring stages; OC=8; self-collision (CHAIN 2) with R = 1
+    # 1+1 warps, one ragged sweep, 3 ring stages; OC=8; self-collision (CHAIN 2)
     "a": ((2, 2, 17, 13, 8, True, False, False), r"iterate_split_kernel<7, ?2, ?1, ?1>", ("coll", "self")),
     # 2+2 warps, one ragged sweep, one stage (T=2, the shortest horizon); OC=4; EE goal
     "b": ((2, 2, 50, 2, 4, False, True, False), r"iterate_split_kernel<7, ?1, ?2, ?2>", ("coll", "ee")),
@@ -311,16 +311,16 @@ def test_split_panda_soft_weights(cuda):
     assert int(live.min()) >= 8, "pass 2 saw at most %d live weights" % int(live.min())
 
 
-def test_split_panda_bench_grid_equals_shards(cuda):
-    """Case f: the 1-GPU benchmark grid (1,537 problems x 4 goals, S=512: 6,148 CTAs, 4+4 warps, 4 sweeps) in one launch against
-    its first and last 38 problems launched alone with problem_gid0 (8+8 warps).  A sample's arithmetic does not depend on the CTA
-    shape: per-sample costs are bit-identical; weights, grad and means agree to the rounding of the block sums."""
-    B, G, S, T = 1537, 4, 512, 64
+def _grid_equals_shards(cuda, S, T, samples):
+    """The 1-GPU benchmark grid (1,537 problems x 4 goals: 6,148 CTAs, 4+4 warps) in one launch against its first and last 38
+    problems launched alone with problem_gid0 (8+8 warps).  A sample's arithmetic does not depend on the CTA shape: per-sample
+    costs (and samples, when `samples`) are bit-identical; weights, grad and means agree to the rounding of the block sums."""
+    B, G = 1537, 4
     ops = _ops()
     spec_of, sh, (desc, _), tab, mu0, step = panda_case(cuda, B, G, S, T, 5)
     mu = mu0.clone()
     with expect_kernel(r"iterate_split_kernel<7, ?1, ?4, ?4>"):
-        out = ops.iterate(sh, desc, tab, step, 1, mu, seed=SEED, draw0=DRAW, want_samples=False, want_means_pre=False)
+        out = ops.iterate(sh, desc, tab, step, 1, mu, seed=SEED, draw0=DRAW, want_samples=samples, want_means_pre=False)
     _, goals, spheres = SC.panda_batch(B, G, 5, seed0=0)
     for lo in (0, B - 38):
         hi = lo + 38
@@ -330,11 +330,24 @@ def test_split_panda_bench_grid_equals_shards(cuda):
         shp = ops.make_shape(38, G, 1, S, T, 7, torch.float32, problem_gid0=lo)
         mup = mu0[lo:hi].clone()
         with expect_kernel(r"iterate_split_kernel<7, ?1, ?8, ?8>"):
-            op = ops.iterate(shp, descp, tab, step, 1, mup, seed=SEED, draw0=DRAW, want_means_pre=False)
+            op = ops.iterate(shp, descp, tab, step, 1, mup, seed=SEED, draw0=DRAW, want_samples=samples, want_means_pre=False)
         assert torch.equal(out["costs"][lo:hi], op["costs"]), "problems %d..%d: per-sample costs differ" % (lo, hi - 1)
+        if samples:
+            assert torch.equal(out["samples"][lo:hi], op["samples"]), "problems %d..%d: samples differ" % (lo, hi - 1)
         assert float((out["weights"][lo:hi] - op["weights"]).abs().max()) < 1e-6
         assert float((out["grad"][lo:hi] - op["grad"]).abs().max() / op["grad"].abs().max()) < 1e-5
         assert float((mu[lo:hi] - mup).abs().max() / mup.abs().max()) < 1e-6
+
+
+def test_split_panda_bench_grid_equals_shards(cuda):
+    """Case f: _grid_equals_shards at the benchmark's shape (S=512, T=64: 4 sweeps), per-sample costs."""
+    _grid_equals_shards(cuda, 512, 64, samples=False)
+
+
+def test_split_panda_cta_shapes_agree(cuda):
+    """_grid_equals_shards at a short horizon (S=256, T=8), where the grid's samples (0.7 GB) fit: costs AND samples of the 4+4
+    and the 8+8 warp shapes are bit-identical."""
+    _grid_equals_shards(cuda, 256, 8, samples=True)
 
 
 # ------------------------------------------------------------------------------------------------ state-only form

@@ -1014,40 +1014,3 @@ torch.save(out, sys.argv[1])
         res.append(torch.load(f))
     for k in res[0]:
         assert torch.equal(res[0][k], res[1][k]), k
-
-
-def test_fused_cta_shapes_agree(cuda, tmp_path):
-    """The role-split Panda kernel runs as 4 + 4 warps per CTA for large grids (the C4 benchmark) and as 8 + 8 warps for grids of
-    <= 6,144 CTAs (the per-GPU share of C4 on 8 GPUs).  $SGPMP_SPLIT_CFG is read once per process, so both shapes run in
-    subprocesses on the same inputs, 38 problems (152 particles: fewer would run the cluster kernel, which does not read
-    $SGPMP_SPLIT_CFG), and each subprocess checks which kernel ran: per-sample costs and samples are bit-identical (a sample's
-    arithmetic does not depend on the CTA shape), weights / gradient / means agree to the rounding of the block-wide softmax sum."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = r'''
-import os, sys, torch
-sys.path.insert(0, %r)
-sys.path.insert(0, os.path.join(%r, "tests"))
-import bench
-from test_gpu_fused_shapes import expect_kernel
-dev = torch.device("cuda:0")
-w = bench.workload("panda", 38)
-pl = bench.build_planner(w, 38, dev)
-obs = {"obstacle_spheres": torch.tensor(w["spheres"], dtype=torch.float32, device=dev)}
-with expect_kernel(r"iterate_split_kernel<7, ?1, ?%%s>" %% sys.argv[2].replace(",", ", ?")):
-    r = pl.optimize(opt_iters=1, return_samples=True, **obs)
-torch.save({"means": pl._means.cpu(), "costs": r[4].cpu(), "samples": r[2].cpu(), "grad": r[5].cpu(), "weights": pl._weights_raw.cpu()}, sys.argv[1])
-''' % (root, root)
-    res = []
-    for cfg in ("4,4", "8,8"):
-        f = str(tmp_path / ("cfg%s.pt" % cfg[0]))
-        env = dict(os.environ, SGPMP_SPLIT_CFG=cfg, SGPMP_LOWLAT="0")
-        subprocess.run([sys.executable, "-c", script, f, cfg], check=True, env=env, timeout=300)
-        res.append(torch.load(f))
-    a, b = res
-    assert torch.equal(a["costs"], b["costs"]) and torch.equal(a["samples"], b["samples"])
-    assert float((a["weights"] - b["weights"]).abs().max()) < 1e-6
-    assert float((a["grad"] - b["grad"]).abs().max() / a["grad"].abs().max()) < 1e-5
-    assert float((a["means"] - b["means"]).abs().max() / a["means"].abs().max()) < 1e-6
