@@ -104,7 +104,8 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float* sph = reinterpret_cast<float*>(smem_raw);           // [MAX_SPHERES][8] + coll_const, self_const
     float* rec = sph + SPH_SMEM;                               // [T][REC]
-    float* wsm = rec + (size_t)T * REC;                        // [S] costs -> weights
+    uint4* ptab = reinterpret_cast<uint4*>(rec + (size_t)T * REC);   // [T][NP2] philox_prefix words of this iteration's draw
+    float* wsm = reinterpret_cast<float*>(ptab + (size_t)T * NP2);   // [S] costs -> weights
     float* red = wsm + Spad;                                   // [32]
     float* start = red + 32;                                   // [16] pair-interleaved like the mu block of a record
     float* goal = start + 16;                                  // [16]
@@ -194,6 +195,9 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
             blk[cv + REC_B] = (float)bv_;
             mub_part += mp * bp_ + mv * bv_;
         }
+        if (!eps)          // the sample-invariant Philox rounds of every (t, k), read by both passes
+            for (int k = tid; k < T * NP2; k += BS)
+                ptab[k] = philox_prefix(philox_x((uint32_t)(k / NP2), (uint32_t)(k % NP2)), pgid, key.draw + dro, key);
         const float mub = (float)block_sum_f64(mub_part, red64);
         if (last && A.means_pre)
             for (int k = tid; k < M; k += BS) A.means_pre[(size_t)bp * M + k] = rec[(k / d) * REC + REC_M + 8 + pidx(k % d)];
@@ -205,13 +209,16 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
             if (role == 0) {
               // MM: occupancy-map mode of this sweep — -1 none, 1 byte map, 2 float map (state-only form; a compile-time constant of
               // the time loop instead of a per-step test)
-              auto state_sweep = [&](auto mm_) {
+              // PLAIN: the in-kernel stream and no sample output (every iteration but a last one that writes samples) — a compile-time
+              // constant, so that the step loop carries neither the eps-injection branch nor emit_row
+              auto state_sweep = [&](auto mm_, auto plain_) {
                 constexpr int MM = decltype(mm_)::value;
+                constexpr bool PLAIN = decltype(plain_)::value;
                 const int sl = sw * SW + wa * 32 + lane;
                 const bool valid = sl < ns;
                 const int s0 = valid ? sl : ns - 1;              // idle lanes shadow the last sample, results dropped
                 // ================= state warps =================
-                const uint32_t sgid = A.sample_gid0 + (uint32_t)s0;
+                const uint2 lw = philox_lane(A.sample_gid0 + (uint32_t)s0, pgid, key);
                 F2 yp[NP2], yv[NP2];
 #pragma unroll
                 for (int k = 0; k < NP2; ++k) yp[k] = yv[k] = f2(0.f, 0.f);
@@ -219,7 +226,7 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
                 TrajCostPairs<N, 0> tcm;          // occupancy-map gather of the state warps (planar: obst_map.py:164-182)
                 tcm.begin();
                 auto draw = [&](int t, F2 (&ep)[NP2], F2 (&ev)[NP2]) {
-                    if (eps) {
+                    if (!PLAIN && eps) {
                         const float* r0 = eps + ((size_t)t * d) * S + s0;
 #pragma unroll
                         for (int k = 0; k < NP2; ++k) {
@@ -228,10 +235,11 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
                             ev[k] = f2(r0[(size_t)(N + i0) * S], i1 < N ? r0[(size_t)(N + i1) * S] : 0.f);
                         }
                     } else {
+                        const uint4* pt = ptab + t * NP2;
 #pragma unroll
                         for (int k = 0; k < NP2; ++k) {
-                            if (2 * k + 1 < N) normal_pair_f2<true>(key, (uint32_t)t, (uint32_t)k, sgid, pgid, ep[k], ev[k], dro);
-                            else normal_pair_f2<false>(key, (uint32_t)t, (uint32_t)k, sgid, pgid, ep[k], ev[k], dro);
+                            if (2 * k + 1 < N) normal_pair_f2<true>(philox_finish(pt[k], lw, key), ep[k], ev[k]);
+                            else normal_pair_f2<false>(philox_finish(pt[k], lw, key), ep[k], ev[k]);
                         }
                     }
                 };
@@ -267,7 +275,7 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
                         cst = vfma(dp, dp, vfma(dv, dv, cst));
                         cis = vfma(yp[k], bp_, vfma(yv[k], bv_, cis));
                     }
-                    if (emit && valid) emit_row(0);
+                    if (!PLAIN && emit && valid) emit_row(0);
                 }
                 for (int t0 = 1; t0 < T; t0 += TS) {
                     const uint32_t stg = sc % NSTG, use = sc / NSTG;
@@ -308,7 +316,7 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
                             const F2 x01 = ld_f2(blk + 8 + REC_M) + yp[0];
                             tcm.template map_gather_deferred<MM>(P, sm, lane0(x01), lane1(x01));
                         }
-                        if (emit && valid) emit_row(t);
+                        if (!PLAIN && emit && valid) emit_row(t);
                     }
                     cgp += cgs;
                     if constexpr (NB > 0) mbar_arrive(bar_full(wa, stg));
@@ -361,13 +369,17 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
                     if (last && A.costs) A.costs[(size_t)bp * S + sl] = c;
                 }
               };
-              if constexpr (NB == 0) {
-                  if (!P.has_map) state_sweep(std::integral_constant<int, -1>{});
-                  else if (sm.map_u8) state_sweep(std::integral_constant<int, 1>{});
-                  else state_sweep(std::integral_constant<int, 2>{});
-              } else {
-                  state_sweep(std::integral_constant<int, -1>{});
-              }
+              auto state_sweep_mm = [&](auto plain) {
+                  if constexpr (NB == 0) {
+                      if (!P.has_map) state_sweep(std::integral_constant<int, -1>{}, plain);
+                      else if (sm.map_u8) state_sweep(std::integral_constant<int, 1>{}, plain);
+                      else state_sweep(std::integral_constant<int, 2>{}, plain);
+                  } else {
+                      state_sweep(std::integral_constant<int, -1>{}, plain);
+                  }
+              };
+              if (!eps && !emit) state_sweep_mm(std::true_type{});
+              else state_sweep_mm(std::false_type{});
             } else if constexpr (NB > 0) {
                 // ================= link warps =================
                 // Link warp wb serves state warp wb.  The field sums of the whole sweep stay in registers and reach shared memory
@@ -478,12 +490,13 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
             for (int item = tid; item < n_items; item += BS) {
                 const int t_ = item / NP2, k = item - t_ * NP2;
                 const bool full = 2 * k + 1 < N;
+                const uint4 pre = ptab[item];
                 float a0 = 0, a1 = 0, a2 = 0, a3 = 0;
                 for (int j = 0; j < nnz; ++j) {
                     const int s = nzl[j];
                     const float w = wsm[s];
                     float p0, p1, v0, v1;
-                    normal_pair<float>(key, (uint32_t)t_, (uint32_t)k, full, A.sample_gid0 + (uint32_t)s, pgid, p0, p1, v0, v1, dro);
+                    normal_pair<float>(philox_finish(pre, philox_lane(A.sample_gid0 + (uint32_t)s, pgid, key), key), full, p0, p1, v0, v1);
                     a0 += w * p0; a1 += w * p1; a2 += w * v0; a3 += w * v1;
                 }
                 acc[t_ * d + 2 * k] = a0;
@@ -528,14 +541,15 @@ iterate_split_kernel(const __grid_constant__ CostParams<float> P, const __grid_c
 template <int N, int CHAIN, int NA, int NB>
 static int launch_split_cfg(const sgpmp_shape_t& sh, const CostParams<float>& P, const IterArgs<float>& A, cudaStream_t st) {
     using Cfg = SplitCfg<NA, NB>;
-    constexpr int d = 2 * N, NSTG = SPLIT_NSTG, REC = rec_floats(N);
+    constexpr int d = 2 * N, NSTG = SPLIT_NSTG, REC = rec_floats(N), NP2 = (N + 1) / 2;
     const int T = sh.T, M = T * d, Mpad = (M + 3) & ~3, Spad = (sh.S + 3) & ~3, NCH = (sh.S + 31) >> 5;
     const size_t phase_bytes = ((size_t)Mpad + Spad + ((NCH + 4) & ~3)) * 4;
     size_t uni = phase_bytes > Cfg::pass1_bytes() ? phase_bytes : Cfg::pass1_bytes();
     // the union region is also stg_tmp, the 32-float start / goal staging scratch of the kernel's start-up; the state-only form
     // has no pass-1 region, and with T = 2 and S <= 4 the block phases alone need only 64 or 80 bytes
     if (uni < 32 * sizeof(float)) uni = 32 * sizeof(float);
-    const size_t smem = ((size_t)SPH_SMEM + (size_t)T * REC + Spad + 32 + 32) * sizeof(float) + 32 * sizeof(double) +
+    const size_t smem = ((size_t)SPH_SMEM + (size_t)T * REC + Spad + 32 + 32) * sizeof(float) + (size_t)T * NP2 * sizeof(uint4) +
+                        32 * sizeof(double) +
                         (size_t)(NB ? ((NA * (2 * NSTG + 1) + 1) & ~1) : 0) * sizeof(uint64_t) + ((uni + 15) & ~(size_t)15);
     if (smem > 227 * 1024) return SGPMP_ERR_UNSUPPORTED;
     auto kern = iterate_split_kernel<N, CHAIN, NA, NB>;
