@@ -79,11 +79,9 @@ if __name__ == '__main__':
     torch.cuda.synchronize()
     print(f'plan: {opt_iters + 1} optimize() calls in {(time.time() - t0) * 1e3:.1f} ms; mean cost {costs.mean().item():.4e}')
 
-    # collision check of the final mean trajectories: signed distance of every link origin to every sphere
-    q = planner.particle_means[..., :n_dof].reshape(-1, n_dof).contiguous()
-    pos = ops.fk_link_positions(panda_fk, q)                                           # [NP*T, 11, 3]
-    sph = obs['obstacle_spheres'][0]
-    dist = (pos[:, :, None, :] - sph[None, None, :, :3]).norm(dim=-1) - sph[None, None, :, 3]
-    print('final means: min link-origin clearance to the spheres = %.3f m' % dist.min().item())
-    ee = pos.reshape(-1, traj_len, pos.shape[1], 3)[:, -1, -1]                         # ee_link origin at t = T-1
-    print('final means: EE position error to the target = %s m' % (ee - target_H[0, :3, 3]).norm(dim=-1).cpu().numpy().round(4))
+    # the final plan: the cheapest collision-free particle mean, checked at 8 states inside every interval as well as at the support
+    # states (the planner's own GP interpolation), against the obstacle spheres
+    best = planner.best_plans(n_interp=8, **obs)
+    ee = ops.fk_link_positions(panda_fk, best.plan[-1:, :n_dof].contiguous())[0, -1]       # ee_link origin at t = T-1
+    print('best plan: particle %d, collision-free %s, clearance to the spheres %.3f m, EE position error to the target %.4f m'
+          % (best.particle.item(), bool(best.collision_free), best.clearance.item(), (ee - target_H[0, :3, 3]).norm().item()))

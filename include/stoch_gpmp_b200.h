@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SGPMP_ABI_VERSION 6
+#define SGPMP_ABI_VERSION 7
 
 enum { SGPMP_F32 = 0, SGPMP_F64 = 1 };
 
@@ -62,6 +62,7 @@ enum {
 #define SGPMP_MAX_SPHERES 16
 #define SGPMP_MAX_INTERP 8        /* link interpolation: extra points per link pair */
 #define SGPMP_MAX_LINK_POINTS 48  /* link frames + interpolated points of one field */
+#define SGPMP_MAX_TIME_INTERP 32  /* sgpmp_select_plans: states checked between two support states */
 #define SGPMP_NUM_TERMS 7
 /* total = (((((start + gp) + goal) + self) + coll) + ee) + is  — the order of the shipped cost lists
  * (examples/panda_environment.py:90), then the IS term (planner.py:236) */
@@ -204,6 +205,22 @@ int sgpmp_cost(const sgpmp_shape_t* shape, const sgpmp_cost_desc_t* desc, const 
  * of CostComposite (cost_functions.py:51-52) when checking collision-freeness of final plans. */
 int sgpmp_fk_link_positions(const sgpmp_cost_desc_t* desc, int32_t n_dof, int32_t dtype, int32_t n_cfg,
                             const void* q, void* pos, void* stream);
+
+/* Final plans (no reference counterpart; the reference's _get_traj('best') takes one argmax over the weights of all samples):
+ * a collision check of every particle mean and, per problem, the best collision-free one.  Two launches, no synchronisation.
+ *   means      [B,NP,T,d]; costs [B,NP] the ranking cost of each mean (sgpmp_cost with S = 1 and means == NULL)
+ *   n_interp   m in [0, SGPMP_MAX_TIME_INTERP]: every mean is checked at P = (T-1)(m+1)+1 states; point j lies in interval
+ *              i = j/(m+1) at tau = (j%(m+1)) dt/(m+1) and is the constant-velocity GP prior's interpolation
+ *              x(tau) = Lambda(tau) x_i + Psi(tau) x_{i+1} per DoF (cubic Hermite in (q, qdot)); tau = 0 is x_i itself
+ *   clearance  [B,NP] out: min over the checked states (all but t = 0) of |p - c| - r over the sphere field's points (link-frame
+ *              origins + its link interpolation) and spheres; +inf without a sphere field.  The self-collision field is not checked.
+ *   hits       [B,NP] out: number of checked states whose occupancy-map cell is non-zero; 0 without a map
+ *   particle   [B] out: argmin cost over the feasible particles (hits == 0, clearance >= margin, finite cost), ties to the lowest
+ *              index; with none feasible the argmin over all (NaN last) and ok = 0.   ok [B] out: 1 if the chosen one is feasible
+ *   plan       [B,T,d] out: means[b, particle[b]] bit for bit;  dense [B,P,d] out (may be NULL): its checked states */
+int sgpmp_select_plans(const sgpmp_shape_t* shape, const sgpmp_cost_desc_t* desc, int32_t n_interp, double margin,
+                       const void* means, const void* costs, void* clearance, int32_t* hits, int32_t* particle, int32_t* ok,
+                       void* plan, void* dense, void* stream);
 
 /* K4 — softmax over the S samples of each particle + weighted-mean update
  * (StochGPMP._update_distribution, planner.py:263-275).  means is updated in place;

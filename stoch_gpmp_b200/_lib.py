@@ -19,7 +19,8 @@ MAX_INTERP = 8
 MAX_LINK_POINTS = 48
 NUM_TERMS = 7
 TERM_NAMES = ("start", "gp", "goal", "coll", "is", "self", "ee")
-ABI_VERSION = 6
+ABI_VERSION = 7
+MAX_TIME_INTERP = 32
 
 
 class Shape(C.Structure):
@@ -65,6 +66,7 @@ SIGNATURES = {
     "sgpmp_sample": (C.c_int, [_SP, _vp, _vp, _vp, _u64, _u32, _vp, _vp, _vp]),
     "sgpmp_cost": (C.c_int, [_SP, _DP, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sgpmp_fk_link_positions": (C.c_int, [_DP, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "sgpmp_select_plans": (C.c_int, [_SP, _DP, _i32, _dbl, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sgpmp_update": (C.c_int, [_SP, _dbl, _dbl, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sgpmp_iterate": (C.c_int, [_SP, _DP, _vp, _dbl, _i32, _vp, _u64, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sgpmp_iterate_lowlat": (C.c_int, [_SP, _DP, _vp, _dbl, _i32, _vp, _u64, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -264,6 +264,18 @@ __device__ __forceinline__ void fk_panda_origins(const CostParams<real>& P, cons
     X[5] = px; Y[5] = py; Z[5] = pz;               // ee_link
 }
 
+// Cell of position (x, y) in the occupancy map: X*(1/cell) + offset with two roundings, floor, int, clamp; value = map[iy][ix].
+// The reference clamps ix with shape[0] and iy with shape[1] (obst_map.py:177-178); maps are square here.
+template <typename real>
+__device__ __forceinline__ int map_cell(const CostParams<real>& P, real x, real y) {
+    const real xo = sg_mul_add_2r(x, P.map_inv_cell, P.map_origin_x);
+    const real yo = sg_mul_add_2r(y, P.map_inv_cell, P.map_origin_y);
+    int ix = (int)sg_floor(xo), iy = (int)sg_floor(yo);
+    ix = min(max(ix, 0), P.map_h - 1);
+    iy = min(max(iy, 0), P.map_w - 1);
+    return iy * P.map_w + ix;
+}
+
 template <typename real, int N, int CHAIN = 0>
 struct TrajCost {
     real c_start, c_gp, c_goal, c_coll, c_is, c_self, c_ee;
@@ -403,16 +415,7 @@ struct TrajCost {
         }
     }
 
-    // X*(1/cell) + offset with two roundings, floor, int, clamp; value = map[iy][ix].  The reference clamps ix
-    // with shape[0] and iy with shape[1] (obst_map.py:177-178); maps are square here.
-    __device__ __forceinline__ int map_index(const CostParams<real>& P, real x, real y) const {
-        const real xo = sg_mul_add_2r(x, P.map_inv_cell, P.map_origin_x);
-        const real yo = sg_mul_add_2r(y, P.map_inv_cell, P.map_origin_y);
-        int ix = (int)sg_floor(xo), iy = (int)sg_floor(yo);
-        ix = min(max(ix, 0), P.map_h - 1);
-        iy = min(max(iy, 0), P.map_w - 1);
-        return iy * P.map_w + ix;
-    }
+    __device__ __forceinline__ int map_index(const CostParams<real>& P, real x, real y) const { return map_cell(P, x, y); }
 
     // feed state x_t (t = 0..T-1 in order)
     // brow: b_t = (Sigma^-1 mu)_t of this particle (2N reals, 16-byte aligned when 2N % 4 == 0 rows are padded), or null

@@ -301,6 +301,27 @@ def fk_link_positions(fk, q):
     return pos
 
 
+def select_plans(shape, desc, means, costs, n_interp, margin, want_dense=True):
+    """Collision check of every particle mean at P = (T-1)(n_interp+1)+1 states (support states and the GP prior's interpolation
+    between them) and the cheapest collision-free mean of each problem.  means [B,NP,T,d], costs [B,NP] (the ranking cost).
+    Returns dict(clearance [B,NP], hits [B,NP] int32, particle [B] int32, ok [B] int32, plan [B,T,d], dense [B,P,d] or None)."""
+    lib = _lib.load()
+    B, NP, T, d = shape.B, shape.G * shape.K, shape.T, 2 * shape.n_dof
+    dt, dev = means.dtype, means.device
+    _req(means, "means", None, (B, NP, T, d))
+    _req(costs, "costs", dt, (B, NP))
+    P = (T - 1) * (max(int(n_interp), 0) + 1) + 1          # an n_interp out of range is rejected by the library
+    i32 = dict(dtype=torch.int32, device=dev)
+    out = dict(clearance=torch.empty(B, NP, dtype=dt, device=dev), hits=torch.empty(B, NP, **i32), particle=torch.empty(B, **i32),
+               ok=torch.empty(B, **i32), plan=torch.empty(B, T, d, dtype=dt, device=dev),
+               dense=torch.empty(B, P, d, dtype=dt, device=dev) if want_dense else None)
+    with _on_device(dev):
+        _lib.check(lib.sgpmp_select_plans(C.byref(shape), C.byref(desc), int(n_interp), float(margin), _ptr(means), _ptr(costs),
+                                          _ptr(out["clearance"]), _ptr(out["hits"]), _ptr(out["particle"]), _ptr(out["ok"]),
+                                          _ptr(out["plan"]), _ptr(out["dense"]), _stream()), "sgpmp_select_plans")
+    return out
+
+
 _GPMP_METHODS = {'inverse': _lib.GPMP_INVERSE, 'cholesky': _lib.GPMP_CHOLESKY}
 
 

@@ -19,6 +19,7 @@ Differences from the reference that a user can observe (DESIGN.md §7):
   * samples are materialised lazily: the fused loop only writes the last iteration's samples when asked
     (`optimize(return_samples=...)`); `get_recent_samples()` regenerates them from the RNG counters.
 """
+import collections
 import time
 
 import torch
@@ -33,6 +34,20 @@ def print_info(iteration, max_iterations, start_time_iter, start_time, costs):
           f'| Iter Time: {time.time() - start_time_iter:.3f}'
           f'| Total Time: {time.time() - start_time:.3f} '
           f'| Cost: {costs.sum(-1).mean():.6f}')
+
+
+PlanResult = collections.namedtuple('PlanResult', [
+    'plan',                 # [B,T,d] the chosen particle mean, bit for bit
+    'dense_plan',           # [B,P,d] its P = (T-1)(n_interp+1)+1 checked states; dense_plan[:, ::n_interp+1] == plan
+    'dense_dt',             # time between two dense states: dt / (n_interp+1)
+    'particle',             # [B] index of the chosen particle
+    'cost',                 # [B] its ranking cost
+    'collision_free',       # [B] bool: the chosen particle passed the check (no occupied map cell, clearance >= margin)
+    'clearance',            # [B] its clearance to the obstacle spheres (+inf without a sphere field)
+    'particle_costs',       # [B,NP] ranking cost of every particle mean
+    'particle_clearance',   # [B,NP]
+    'particle_hits',        # [B,NP] checked states in an occupied map cell
+])
 
 
 def prior_blocks(T, dt, sigma_start, sigma_gp, sigma_goal):
@@ -520,6 +535,43 @@ class StochGPMPBatch:
             ind = self._weights.argmax()
             return self.state_samples.reshape(-1, self.num_samples, self.traj_len, self.d_state_opt)[ind].clone()
         raise ValueError('Unidentified sampling mode in get_next_action')
+
+    def best_plans(self, n_interp=8, margin=0.0, **observation):
+        """The final step of planning: one plan per problem, with a yes/no answer on whether it is collision-free.  No reference
+        counterpart (DESIGN.md §7).  Returns a PlanResult (fields above; StochGPMP drops the B axis).
+
+        Works on the CURRENT particle means (`particle_means`, i.e. after the last update), not on the pre-update means that
+        optimize() returns.  Every mean is checked at its support states t >= 1 and at n_interp states inside every interval: the
+        constant-velocity GP prior's own interpolation (cubic Hermite in (q, qdot)), so the check holds for the trajectory model the
+        planner optimises, not only at its support states.  The obstacle spheres of `observation` (as optimize() takes them) are
+        checked geometrically: clearance is the least |p - c| - r over the sphere field's points (link-frame origins and its link
+        interpolation) and spheres, whatever the field type.  Occupancy maps of the cost are checked cell by cell.  The
+        self-collision field is NOT checked: its RBF over all link pairs, adjacent links included, defines no distance to hold
+        against a margin.
+
+        A particle is collision-free when no checked state lies in an occupied map cell and its clearance is >= margin (in
+        metres).  The plan of a problem is its cheapest collision-free particle (ties to the lowest index); with none, the
+        cheapest particle overall (NaN costs last), with collision_free False.  The ranking cost is CostComposite.eval of the
+        mean without the importance-sampling term."""
+        low = self._lowered
+        if low is None:
+            raise NotImplementedError("best_plans needs a CostComposite (cost=...)")
+        if low.custom:
+            raise NotImplementedError("best_plans ranks the means with the CUDA cost kernel; user-defined cost objects (%s) are not "
+                                      "supported" % ", ".join(type(c).__name__ for c in low.custom))
+        B, NP = self.num_problems, self.num_particles
+        sh = self._shape(S=1)
+        desc = low.desc(0.0, observation.get('obstacle_spheres', None))
+        # [B,NP,T,d] is the S-minor sample layout [B,NP,T,d,1]; means=None drops the IS term; the goal of particle p is p // K
+        costs = ops.cost(sh, desc, None, self._means.unsqueeze(-1), None).reshape(B, NP)
+        r = ops.select_plans(sh, desc, self._means, costs, n_interp, margin)
+        particle = r['particle'].long()
+        pick = particle.unsqueeze(1)
+        o = self._out
+        return PlanResult(plan=o(r['plan']), dense_plan=o(r['dense']), dense_dt=self.dt / (n_interp + 1), particle=o(particle),
+                          cost=o(costs.gather(1, pick).squeeze(1)), collision_free=o(r['ok'].bool()),
+                          clearance=o(r['clearance'].gather(1, pick).squeeze(1)), particle_costs=o(costs),
+                          particle_clearance=o(r['clearance']), particle_hits=o(r['hits']))
 
 
 class StochGPMP(StochGPMPBatch):
